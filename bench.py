@@ -3,6 +3,7 @@
 
   python bench.py [--gpus N] [--steps K] [--warmup W]            # this repo's CUDA path (one JSON line on rank 0)
   python bench.py --impl reference [...]                          # the reference's own CPU formulation, same metric
+  python bench.py --dump-outputs DIR [...]                        # + the last timed step's top-k as DIR/<name>.npy
 
 Workload (config.workload): a RESIDENT SHARD of BASELINE configs[1] -- "1M pages x 1024 patches x 128-d bf16, batch-32
 queries" needs 262 GB, more than one B200's HBM (SURVEY F7) -- i.e. `--pages` pages per GPU (default 524288 = 137.4 GB of
@@ -517,8 +518,9 @@ def run_gpu(args):
     free_b, total_b = torch.cuda.mem_get_info(device)
     n_pages = args.pages
     budget_pages = int((free_b - (24 << 30)) // (P_PATCH * 256))  # leave 24 GB for scratch, sub-shards and the FDE matrix
-    if n_pages > budget_pages:
-        n_pages = max(4096, budget_pages // 4096 * 4096)
+    if n_pages > budget_pages:  # a smaller shard would be a different workload with different inputs: say so instead
+        raise SystemExit(f"--pages {n_pages} does not fit in the {free_b / 2**30:.1f} GiB free on cuda:{local_rank} "
+                         f"(24 GiB stay free for the other legs): pass --pages {max(4096, budget_pages // 4096 * 4096)} or fewer")
     rows = n_pages * P_PATCH
     t_build0 = time.perf_counter()
 
@@ -669,6 +671,10 @@ def run_gpu(args):
     clocks = sampler.stop(t_host0, t_host1)
     ms_total = ev0.elapsed_time(ev1)
     launches = idx.launch_count() - launches0
+    # what a caller of the timed path receives from its last step (identical on every rank at N > 1)
+    last_out = out_dev[(args.steps - 1) & 1] if world > 1 else out_dev[0]
+    timed_outputs = {"topk_scores": last_out[0].cpu().numpy(), "topk_ids": last_out[1].cpu().numpy(),
+                     "topk_counts": last_out[2].cpu().numpy()} if args.dump_outputs and rank == 0 else None
     score_ms = idx.score_times_ms(min(args.steps, 256))  # scoring kernels only, events recorded inside the timed region
     score_ms_avg = sum(score_ms) / len(score_ms)
     per_rank = None
@@ -857,6 +863,8 @@ def run_gpu(args):
             cpu["topk_match"] = {"error": repr(e)[:200]}
         del pages_np
 
+    if timed_outputs is not None:
+        dump_outputs(args.dump_outputs, timed_outputs)
     if rank == 0:
         cfg = workload_config(args, n_pages)
         cfg["placement"] = placement
@@ -1002,6 +1010,19 @@ def two_stage_leg(args, idx, packed, n_pages, topic_pages, anchors, sharded, wor
     return out
 
 
+def dump_outputs(out_dir, arrays, limit_bytes=64 << 20):
+    """Write each array as out_dir/<name>.npy: float32 / float64 as they are, integers as float64 (exact below 2^53)."""
+    import numpy as np
+
+    arrays = {name: a if a.dtype in (np.float32, np.float64) else a.astype(np.float64) for name, a in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    if total > limit_bytes:
+        raise ValueError(f"{total} bytes of outputs exceed the {limit_bytes}-byte dump limit")
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
+
+
 def main():
     import faulthandler
 
@@ -1028,7 +1049,13 @@ def main():
     ap.add_argument("--check-pages", type=int, default=256, help="pages per rank in the multi-GPU oracle check")
     ap.add_argument("--settle-steps", type=int, default=12, help="untimed steps before the timed region (>= warmup): power-capped clocks settle")
     ap.add_argument("--placement", choices=["equal", "speed"], default=os.environ.get("B200MS_PLACEMENT", "equal"))
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write the top-k of the last one (scores, ids, "
+                    "counts) as DIR/<name>.npy, so that two builds can be compared on the same seeded inputs")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs applies to the b200 path")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
     if args.impl == "reference":
         run_reference(args)

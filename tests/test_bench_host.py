@@ -6,6 +6,7 @@ import subprocess
 import sys
 
 import numpy as np
+import pytest
 import torch
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -53,3 +54,15 @@ def test_defaults_finish_within_minutes():
     assert 'ap.add_argument("--gpus", type=int, default=1)' in src
     assert 'ap.add_argument("--pages", type=int, default=524288' in src  # the largest resident shard (SURVEY 8d)
     assert np.prod([524288, 1024, 256]) < 180e9
+
+
+def test_dump_outputs_writes_float_arrays_and_enforces_the_size_limit(tmp_path):
+    ids = np.array([[3, 2 ** 40 + 1]], dtype=np.int64)
+    scores = np.array([[1.5, -0.25]], dtype=np.float32)
+    bench.dump_outputs(str(tmp_path / "out"), {"topk_scores": scores, "topk_ids": ids})
+    got_s, got_i = np.load(tmp_path / "out" / "topk_scores.npy"), np.load(tmp_path / "out" / "topk_ids.npy")
+    assert got_s.dtype == np.float32 and np.array_equal(got_s, scores)
+    assert got_i.dtype == np.float64 and np.array_equal(got_i.astype(np.int64), ids)
+    with pytest.raises(ValueError):
+        bench.dump_outputs(str(tmp_path / "big"), {"x": np.zeros((1 << 20) + 1, dtype=np.float64)}, limit_bytes=8 << 20)
+    assert not (tmp_path / "big").exists()

@@ -107,8 +107,8 @@ def test_bf16_config0_shape_single_query():
     np.testing.assert_allclose(ts[0], os_, rtol=2e-5)
 
 
-def test_bf16_golden_fixture_from_score_multi_vector(golden_dir):
-    fm = np.load(os.path.join(golden_dir, "float_maxsim.npz"))
+def test_bf16_golden_fixture_from_score_multi_vector(float_maxsim):
+    fm = float_maxsim
     # case D is bf16-valued (what ColQwen emits), so bf16 storage is lossless and the port's scores are the target
     idx = MaxSimIndex(dtype="bf16")
     idx.add_pages(list(fm["d_pages"]))
@@ -575,11 +575,11 @@ def test_fp8_matches_oracle(n_q):
 
 # ------------------------------------------------------------------------------------------------ zero_pad_compat (SURVEY App. A.2)
 @pytest.mark.parametrize("case,batch", [("b", 128), ("c", 3)])
-def test_zero_pad_compat_matches_score_multi_vector_golden(golden_dir, case, batch):
+def test_zero_pad_compat_matches_score_multi_vector_golden(float_maxsim, case, batch):
     """Product option zero_pad_compat=<batch size> reproduces colpali_engine score_multi_vector's padding quirk (a page
     shorter than the longest of its batch scores max(true, 0) per token): golden cases B (one 128-batch) and C
     (batch_size=3) were produced by the transformers port of score_multi_vector (tests/golden/make_golden.py)."""
-    fm = np.load(os.path.join(golden_dir, "float_maxsim.npz"))
+    fm = float_maxsim
     lens = fm["b_lens"].tolist()
     off = orc.page_offsets(lens)
     pages = [fm["b_rows"][off[i]:off[i + 1]] for i in range(len(lens))]
@@ -631,10 +631,10 @@ def test_zero_pad_compat_rerank_batches_candidates_like_the_reference():
         np.testing.assert_allclose(ts[row].cpu().numpy(), [w[order[j]] for j in exp], rtol=3e-5, atol=1e-6)
 
 
-def test_zero_pad_compat_rerank_matches_port_golden(golden_dir):
+def test_zero_pad_compat_rerank_matches_port_golden(float_maxsim):
     """Golden case E (produced by the transformers port of score_multi_vector): the reference's rerank call, candidates in
     first-stage order -- b200ms_rerank_batch_device with zero_pad_compat=128 returns the port's scores and ranking."""
-    fm = np.load(os.path.join(golden_dir, "float_maxsim.npz"))
+    fm = float_maxsim
     lens = fm["e_lens"].tolist()
     off = orc.page_offsets(lens)
     pages = [fm["e_rows"][off[i]:off[i + 1]] for i in range(len(lens))]

@@ -19,8 +19,8 @@ def sp(golden_dir):
 
 
 @pytest.fixture(scope="module")
-def fm(golden_dir):
-    return np.load(os.path.join(golden_dir, "float_maxsim.npz"))
+def fm(float_maxsim):
+    return float_maxsim
 
 
 def test_sign_pack_matches_reference_fast_ops(sp):

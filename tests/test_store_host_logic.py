@@ -258,63 +258,61 @@ def test_batch_query_mask_search_and_chunks_are_one_critical_section():
     assert idx.bad == 0
 
 
-@pytest.mark.skipif(not __import__("os").path.exists("/root/reference/core/vector_store/dual_multivector_store.py"),
-                    reason="needs the reference checkout (build container only)")
-def test_reference_dual_multivector_store_runs_unmodified_over_this_store():
-    """SURVEY row a-11: the reference's own DualMultiVectorStore (core/vector_store/dual_multivector_store.py), executed
-    unmodified, with two B200MultiVectorStore instances as its fast / slow members.  Only its sibling imports -- the Postgres and
-    Turbopuffer stores, which need psycopg / turbopuffer -- are replaced by empty placeholder classes (they are used as type
-    annotations there); every method the dual store calls on its members is this repo's."""
-    import importlib.util
-    import sys
-    import types
+def test_reference_dual_store_calls_replay_over_this_store(golden_dir):
+    """SURVEY row a-11: the reference's DualMultiVectorStore (core/vector_store/dual_multivector_store.py) drives two stores as
+    its fast / slow members.  tests/golden/dual_store_calls.json holds every member call it made (method, positional and
+    keyword arguments) and every member attribute it read in this scenario (tests/golden/make_golden.py ran it over
+    recording members).  Replayed as recorded on two B200MultiVectorStore instances -- the calls of one operation awaited
+    together, as the dual store does -- each call is accepted, returns what the dual store unpacks, and the scenario holds."""
+    import json
+    import os
 
-    ref = "/root/reference"
-    saved = {k: sys.modules.get(k) for k in ("core", "core.vector_store", "core.vector_store.base_vector_store",
-                                             "core.vector_store.fast_multivector_store", "core.vector_store.multi_vector_store",
-                                             "core.models", "core.models.chunk", "core.vector_store.dual_multivector_store")}
-    try:
-        def load(name, path, is_pkg=False):
-            spec = importlib.util.spec_from_file_location(name, path, submodule_search_locations=[path.rsplit("/", 1)[0]] if is_pkg else None)
-            mod = importlib.util.module_from_spec(spec)
-            sys.modules[name] = mod
-            spec.loader.exec_module(mod)
-            return mod
+    with open(os.path.join(golden_dir, "dual_store_calls.json")) as f:
+        ops = json.load(f)["operations"]
+    members = {"fast": B200MultiVectorStore(index=OracleIndex(), mode="binary", auto_initialize=False, uri="b200://fast"),
+               "slow": B200MultiVectorStore(index=OracleIndex(), mode="binary", auto_initialize=False, uri="b200://slow",
+                                            storage="the-storage")}
+    rng = np.random.default_rng(8)
+    chunks = [chunk(f"d{i // 2}", i % 2, rng.standard_normal((3, 128)).astype(np.float32), content=f"c{i}", meta={"i": i})
+              for i in range(8)]
+    refs = {"chunks": chunks, "query": chunks[5].embedding}
 
-        for pkg in ("core", "core.vector_store", "core.models"):
-            m = types.ModuleType(pkg)
-            m.__path__ = [f"{ref}/{pkg.replace('.', '/')}"]
-            sys.modules[pkg] = m
-        load("core.models.chunk", f"{ref}/core/models/chunk.py")
-        load("core.vector_store.base_vector_store", f"{ref}/core/vector_store/base_vector_store.py")
-        for name, cls in (("fast_multivector_store", "FastMultiVectorStore"), ("multi_vector_store", "MultiVectorStore")):
-            stub = types.ModuleType(f"core.vector_store.{name}")
-            setattr(stub, cls, type(cls, (), {}))
-            sys.modules[f"core.vector_store.{name}"] = stub
-        dual_mod = load("core.vector_store.dual_multivector_store", f"{ref}/core/vector_store/dual_multivector_store.py")
-        RefChunk = sys.modules["core.models.chunk"].DocumentChunk
+    def arg(a):
+        if isinstance(a, dict):
+            return refs[a["ref"]]
+        if isinstance(a, list):  # chunk identifiers are (document_id, chunk_number) tuples
+            return [tuple(x) if isinstance(x, list) else x for x in a]
+        return a
 
-        fast = B200MultiVectorStore(index=OracleIndex(), mode="binary", auto_initialize=False, uri="b200://fast")
-        slow = B200MultiVectorStore(index=OracleIndex(), mode="binary", auto_initialize=False, uri="b200://slow", storage="the-storage")
-        dual = dual_mod.DualMultiVectorStore(fast_store=fast, slow_store=slow)
-        assert dual.initialize() is True and dual.uri == "b200://slow" and dual.storage == "the-storage"
-        rng = np.random.default_rng(8)
-        chunks = [RefChunk(document_id=f"d{i // 2}", content=f"c{i}", embedding=rng.standard_normal((3, 128)).astype(np.float32),
-                           chunk_number=i % 2, metadata={"i": i}) for i in range(8)]
-        ok, ids, metrics = run(dual.store_embeddings(chunks, app_id="app"))
-        assert ok and ids == [f"d{i // 2}-{i % 2}" for i in range(8)] and metrics["mode"] == "dual" and {"fast", "slow"} <= set(metrics)
-        assert len(fast.catalog) == len(slow.catalog) == 8
-        res = run(dual.query_similar(chunks[5].embedding, 3, None, "app"))
-        assert (res[0].document_id, res[0].chunk_number) == ("d2", 1) and res[0].metadata == {"i": 5}
-        got = run(dual.get_chunks_by_id([("d1", 0), ("zz", 0)], "app"))
-        assert [(c.document_id, c.chunk_number) for c in got] == [("d1", 0)]
-        assert run(dual.delete_chunks_by_document_id("d2", "app")) is True
-        assert fast.catalog.pages_of("d2") == [] and slow.catalog.pages_of("d2") == []
-        assert all(r.document_id != "d2" for r in run(dual.query_similar(chunks[5].embedding, 8, None, "app")))
-        dual.close()
-    finally:
-        for k, v in saved.items():
-            if v is None:
-                sys.modules.pop(k, None)
+    async def replay(calls):
+        out, pending = [None] * len(calls), []
+        for j, c in enumerate(calls):
+            m = members[c["member"]]
+            if "attribute" in c:
+                out[j] = getattr(m, c["attribute"])
+                continue
+            r = getattr(m, c["method"])(*[arg(a) for a in c["args"]], **{k: arg(v) for k, v in c["kwargs"].items()})
+            if asyncio.iscoroutine(r):
+                pending.append((j, r))
             else:
-                sys.modules[k] = v
+                out[j] = r
+        for (j, _), r in zip(pending, await asyncio.gather(*(r for _, r in pending))):
+            out[j] = r
+        return [(c["member"], res) for c, res in zip(calls, out)]
+
+    got = {op["label"]: run(replay(op["calls"])) for op in ops}
+    assert got["initialize"] == [("fast", True), ("slow", True)]
+    assert got["uri"] == [("slow", "b200://slow")] and got["storage"] == [("slow", "the-storage")]
+    assert [m for m, _ in got["store_embeddings"]] == ["fast", "slow"]
+    for _, (ok, ids, metrics) in got["store_embeddings"]:  # the dual store unpacks (success, ids, metrics) from each member
+        assert ok is True and ids == [f"d{i // 2}-{i % 2}" for i in range(8)] and isinstance(metrics, dict) and metrics
+    assert len(members["fast"].catalog) == len(members["slow"].catalog) == 8
+    [(m, res)] = got["query_similar"]
+    assert m == "slow" and len(res) == 3 and (res[0].document_id, res[0].chunk_number) == ("d2", 1) and res[0].metadata == {"i": 5}
+    [(m, res)] = got["get_chunks_by_id"]
+    assert m == "slow" and [(c.document_id, c.chunk_number) for c in res] == [("d1", 0)]
+    assert got["delete_chunks_by_document_id"] == [("fast", True), ("slow", True)]
+    assert members["fast"].catalog.pages_of("d2") == [] and members["slow"].catalog.pages_of("d2") == []
+    [(m, res)] = got["query_similar_after_delete"]
+    assert m == "slow" and len(res) == 6 and all(r.document_id != "d2" for r in res)
+    assert [m for m, _ in got["close"]] == ["fast", "slow"]
