@@ -17,13 +17,11 @@
 // Bound: tensor pipe / expansion ALU, ~0.5 patch rows per clock per SM (vs 0.18 for the POPC kernel at one query).
 #include "common.cuh"
 #include "ptx.cuh"
+#include "umma_tile.cuh"
 
 namespace bms {
 
 constexpr int kBThreads = 384;
-constexpr int kBAccum = 4;
-constexpr uint32_t kBTileBytes = 128 * 128;  // one int8 tile: 128 rows x 128 B
-constexpr uint32_t kBSmemLimit = 232448;
 
 // ------------------------------------------------------------------ query side: bits -> +-1 int8 rows + token constants
 __global__ void __launch_bounds__(256)
@@ -47,131 +45,55 @@ b1_query_expand_kernel(const uint8_t* __restrict__ q_bits /*[rows,16]*/, const i
   }
 }
 
-// ------------------------------------------------------------------ tile iterator shared by all warp roles
-struct TileIter {
-  int u, t, n_tiles, c0, c1;
-  __device__ __forceinline__ void load(const int32_t* us, const int32_t* ue, int n_units) {
-    n_tiles = 0;
-    while (u < n_units) {
-      c0 = __ldg(us + u);
-      c1 = __ldg(ue + u);
-      n_tiles = (c1 - c0 + 3) >> 2;
-      if (n_tiles > 0) break;
-      u += gridDim.x;
-    }
-    t = 0;
-  }
-  __device__ __forceinline__ bool valid(int n_units) const { return u < n_units; }
-  __device__ __forceinline__ void next(const int32_t* us, const int32_t* ue, int n_units) {
-    if (++t == n_tiles) {
-      u += gridDim.x;
-      load(us, ue, n_units);
-    }
-  }
-  __device__ __forceinline__ int64_t row0() const { return int64_t(c0 + 4 * t) * kGroup; }
-};
-
-__device__ __forceinline__ int chunk_max_i(const uint32_t (&v)[32]) {
-  int a = int(v[0]), b = int(v[1]);
-#pragma unroll
-  for (int i = 2; i < 30; i += 4) {
-    a = imax3(a, int(v[i]), int(v[i + 1]));
-    b = imax3(b, int(v[i + 2]), int(v[i + 3]));
-  }
-  a = imax3(a, int(v[30]), int(v[31]));
-  return max(a, b);
-}
-
-// SPLIT4 (NM == 1, a single 32-token group): the query rows are replicated into all four 32-lane quadrants of the tile, so
-// each epilogue warp reduces ONE 32-column chunk of the accumulator instead of warp 0 walking all four serially (with one
-// tile every ~256 cycles the single-warp epilogue latency, ~600+ cycles per tile, was the measured limiter); the four chunk
-// maxima meet in shared memory once per tile and warp 0 applies the page logic.
-template <int NM, bool SPLIT4>
+template <int NM>
 __global__ void __launch_bounds__(kBThreads, 1)
 maxsim_b1_umma_kernel(const uint4* __restrict__ rows, int64_t n_rows, const __grid_constant__ CUtensorMap tmap_q,
                       const int32_t* __restrict__ tok_const, const int32_t* __restrict__ chunk_page,
                       const int32_t* __restrict__ unit_start, const int32_t* __restrict__ unit_end, int n_units,
                       int m_tile_base, int n_groups_real, int32_t* __restrict__ group_scores, int64_t ld, int num_stages) {
   extern __shared__ uint8_t smem_raw[];
-  uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
-  uint8_t* smem_q = smem;
-  uint8_t* smem_st = smem + NM * kBTileBytes;
-  uint64_t* bars = reinterpret_cast<uint64_t*>(smem_st + size_t(num_stages) * kBTileBytes);
-  uint64_t* full = bars;         // [num_stages] expanders -> MMA   (4 arrivals: one per expander warp)
-  uint64_t* empty = bars + 16;   // [num_stages] MMA -> expanders
-  uint64_t* tfull = bars + 32;   // [kBAccum]    MMA -> epilogue
-  uint64_t* tempty = bars + 40;  // [kBAccum]    epilogue -> MMA
-  uint64_t* qfull = bars + 48;
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + 56);
-  int* slab = reinterpret_cast<int*>(bars + 64);  // SPLIT4: [2][4][32] chunk maxima exchanged between the epilogue warps
-
+  const TileSmem sm = carve_tile_smem(smem_raw, NM * kSubtileBytes, kSubtileBytes, num_stages);
   const int warp = threadIdx.x >> 5;
   const int lane = threadIdx.x & 31;
-
-  if (warp == 0 && lane == 0) {
-    prefetch_tmap(&tmap_q);
-    for (int i = 0; i < num_stages; ++i) {
-      mbar_init(&full[i], 4);
-      mbar_init(&empty[i], 1);
-    }
-    for (int i = 0; i < kBAccum; ++i) {
-      mbar_init(&tfull[i], 1);
-      mbar_init(&tempty[i], 4);
-    }
-    mbar_init(qfull, 1);
-    fence_mbar_init();
-  }
-  if (warp == 2) tmem_alloc_512(tmem_slot);
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  const uint32_t tmem_base = *tmem_slot;
+  // full: one arrive per expander warp
+  const uint32_t tmem_base = tile_prologue<false>(sm, warp, &tmap_q, nullptr, num_stages, 4, kNumAccum, 4);
 
   if (warp == 0) {
     // ================================================================ query tiles via TMA (+-1 int8, SWIZZLE_128B)
     if (lane == 0) {
       const uint64_t pol_q = policy_evict_last();
-      mbar_expect_tx(qfull, NM * kBTileBytes);
-      if constexpr (SPLIT4) {  // tmap_q has 32-row boxes here: the same 32 token rows land in all four row quarters
+      mbar_expect_tx(sm.qfull, NM * kSubtileBytes);
 #pragma unroll
-        for (int j = 0; j < 4; ++j) tma_load_2d(&tmap_q, qfull, smem_q + j * 4096, 0, m_tile_base * kTileM, pol_q);
-      } else {
-#pragma unroll
-        for (int m = 0; m < NM; ++m) tma_load_2d(&tmap_q, qfull, smem_q + m * kBTileBytes, 0, (m_tile_base + m) * kTileM, pol_q);
-      }
+      for (int m = 0; m < NM; ++m) tma_load_2d(&tmap_q, sm.qfull, sm.q + m * kSubtileBytes, 0, (m_tile_base + m) * kTileM, pol_q);
     }
   } else if (warp == 1) {
     // ================================================================ MMA issuer (kind::i8, 4 K-steps of 32 per tile)
     constexpr uint32_t idesc = umma_idesc(1, kTileM, kTileN);
-    constexpr uint32_t kTileDesc = kBTileBytes >> 4;
-    mbar_wait(qfull, 0);
+    constexpr uint32_t kTileDesc = kSubtileBytes >> 4;
+    mbar_wait(sm.qfull, 0);
     tc_fence_after();
-    const uint64_t a_desc0 = umma_desc_kmajor_sw128(smem_u32(smem_q));
-    const uint64_t b_desc0 = umma_desc_kmajor_sw128(smem_u32(smem_st));
+    const uint64_t a_desc0 = umma_desc_kmajor_sw128(smem_u32(sm.q));
+    const uint64_t b_desc0 = umma_desc_kmajor_sw128(smem_u32(sm.st));
     int stage = 0;
     uint32_t phase = 0, seq = 0;
-    TileIter it;
-    it.u = blockIdx.x;
-    it.load(unit_start, unit_end, n_units);
-    for (; it.valid(n_units); it.next(unit_start, unit_end, n_units)) {
-      mbar_wait(&full[stage], phase);
+    UnitWalk it;
+    for (it.init(blockIdx.x, gridDim.x, unit_start, unit_end, n_units); it.valid(n_units);
+         it.next(unit_start, unit_end, n_units)) {
+      mbar_wait(&sm.full[stage], phase);
       tc_fence_after();
       const uint64_t bd = b_desc0 + uint64_t(uint32_t(stage) * kTileDesc);
 #pragma unroll 1
       for (int m = 0; m < NM; ++m, ++seq) {
-        const uint32_t buf = seq & (kBAccum - 1);
-        mbar_wait(&tempty[buf], ((seq >> 2) & 1) ^ 1);
+        const uint32_t buf = seq & (kNumAccum - 1);
+        mbar_wait(&sm.tempty[buf], ((seq >> 2) & 1) ^ 1);
         tc_fence_after();
         if (elect_one()) {
-          const uint32_t d_tmem = tmem_base + buf * kTileN;
-          const uint64_t ad = a_desc0 + uint64_t(uint32_t(m) * kTileDesc);
-#pragma unroll
-          for (int ks = 0; ks < 4; ++ks) umma_ss<1>(d_tmem, ad + ks * 2, bd + ks * 2, idesc, ks != 0);
-          umma_commit(&tfull[buf]);
+          umma_tile<1>(tmem_base + buf * kTileN, a_desc0 + uint64_t(uint32_t(m) * kTileDesc), bd, idesc);
+          umma_commit(&sm.tfull[buf]);
         }
         __syncwarp();
       }
-      if (elect_one()) umma_commit(&empty[stage]);
+      if (elect_one()) umma_commit(&sm.empty[stage]);
       __syncwarp();
       if (++stage == num_stages) {
         stage = 0;
@@ -183,17 +105,16 @@ maxsim_b1_umma_kernel(const uint4* __restrict__ rows, int64_t n_rows, const __gr
     const int r = (warp - 8) * 32 + lane;  // row of the tile this thread owns
     const uint32_t row_off = uint32_t(r >> 3) * 1024u + uint32_t(r & 7) * 128u;
     const uint32_t sw = uint32_t(r & 7);
-    TileIter cur, pf;
-    cur.u = pf.u = blockIdx.x;
-    cur.load(unit_start, unit_end, n_units);
-    pf = cur;
+    UnitWalk cur;
+    cur.init(blockIdx.x, gridDim.x, unit_start, unit_end, n_units);
+    UnitWalk pf = cur;
     constexpr int kRing = 8;
     uint4 ring[kRing];  // loads of the next 8 tiles stay in flight while the current one is expanded (DRAM latency >> tile time)
 #pragma unroll
     for (int i = 0; i < kRing; ++i) {
       ring[i] = make_uint4(0, 0, 0, 0);
       if (pf.valid(n_units)) {
-        const int64_t row = pf.row0() + r;
+        const int64_t row = int64_t(pf.chunk()) * kGroup + r;
         if (row < n_rows) ring[i] = __ldg(rows + row);
         pf.next(unit_start, unit_end, n_units);
       }
@@ -207,12 +128,12 @@ maxsim_b1_umma_kernel(const uint4* __restrict__ rows, int64_t n_rows, const __gr
         const uint4 mine = ring[i];
         ring[i] = make_uint4(0, 0, 0, 0);
         if (pf.valid(n_units)) {
-          const int64_t row = pf.row0() + r;
+          const int64_t row = int64_t(pf.chunk()) * kGroup + r;
           if (row < n_rows) ring[i] = __ldg(rows + row);
           pf.next(unit_start, unit_end, n_units);
         }
-        mbar_wait(&empty[stage], phase ^ 1);
-        const uint32_t tile = smem_u32(smem_st) + uint32_t(stage) * kBTileBytes + row_off;  // 32-bit shared address: st.shared, not generic ST
+        mbar_wait(&sm.empty[stage], phase ^ 1);
+        const uint32_t tile = smem_u32(sm.st) + uint32_t(stage) * kSubtileBytes + row_off;  // 32-bit shared address: st.shared, not generic ST
         const uint32_t words[4] = {mine.x, mine.y, mine.z, mine.w};
 #pragma unroll
         for (int w = 0; w < 4; ++w) {
@@ -234,7 +155,7 @@ maxsim_b1_umma_kernel(const uint4* __restrict__ rows, int64_t n_rows, const __gr
         }
         fence_proxy_async_smem();  // generic-proxy stores -> visible to the tensor core's async-proxy reads
         __syncwarp();
-        if (lane == 0) mbar_arrive(&full[stage]);
+        if (lane == 0) mbar_arrive(&sm.full[stage]);
         if (++stage == num_stages) {
           stage = 0;
           phase ^= 1;
@@ -246,186 +167,79 @@ maxsim_b1_umma_kernel(const uint4* __restrict__ rows, int64_t n_rows, const __gr
     // ================================================================ epilogue (one warpgroup owns every query tile)
     const int quad = warp & 3;
     const uint32_t lane_base = tmem_base + (uint32_t(quad * 32) << 16);
-    if constexpr (SPLIT4) {
-      const int group = m_tile_base * 4;  // the one real group; every quadrant holds a copy of its 32 token rows
-      const int cn = __ldg(tok_const + int64_t(m_tile_base) * kTileM + lane);
-      int rm = 0, cp = -1;
-      uint32_t seq = 0;
-      int last_u = -1;
-      TileIter it;
-      it.u = blockIdx.x;
-      it.load(unit_start, unit_end, n_units);
-      for (; it.valid(n_units); it.next(unit_start, unit_end, n_units), ++seq) {
-        const uint32_t buf = seq & (kBAccum - 1);
-        mbar_wait(&tfull[buf], (seq >> 2) & 1);
-        tc_fence_after();
-        uint32_t va[32];
-        tmem_ld_32x32(lane_base + buf * kTileN + quad * 32, va);  // chunk `quad` of this warp's own copy of the rows
-        tmem_ld_wait();
-        tc_fence_before();
-        __syncwarp();
-        if (lane == 0) mbar_arrive(&tempty[buf]);
-        int* sl = slab + (seq & 1) * 128;
-        sl[quad * 32 + lane] = chunk_max_i(va);
-        asm volatile("bar.sync 1, 128;" ::: "memory");  // the four epilogue warps
-        if (quad == 0) {
-          if (it.u != last_u) {
-            if (last_u >= 0 && cp >= 0) {
-              const int s2 = warp_sum(rm + cn);
-              if (lane == 0) group_scores[int64_t(group) * ld + cp] = s2;
-            }
-            cp = -1;
-            last_u = it.u;
-          }
-          const int cb = it.c0 + 4 * it.t;
-#pragma unroll
-          for (int j = 0; j < 4; ++j) {
-            if (cb + j >= it.c1) break;
-            const int pgj = __ldg(chunk_page + cb + j);
-            const int v = sl[j * 32 + lane];
-            if (pgj != cp) {
-              if (cp >= 0) {
-                const int s2 = warp_sum(rm + cn);
-                if (lane == 0) group_scores[int64_t(group) * ld + cp] = s2;
-              }
-              cp = pgj;
-              rm = v;
-            } else {
-              rm = max(rm, v);
-            }
-          }
-        }
-      }
-      if (quad == 0 && cp >= 0) {
-        const int s2 = warp_sum(rm + cn);
-        if (lane == 0) group_scores[int64_t(group) * ld + cp] = s2;
-      }
-    } else {
-    int runmax[NM], cur_page[NM], cnst[NM];
+    // one closed (group, page) run: the per-token constant, the 32-token sum, one store by lane 0
+    const auto store = [&](int group, int cn, int page, int rm) {
+      const int s = warp_sum(rm + cn);
+      if (lane == 0) group_scores[int64_t(group) * ld + page] = s;
+    };
+    PageRun<int> runs[NM];
+    int cnst[NM];
 #pragma unroll
     for (int m = 0; m < NM; ++m) {
       const int group = (m_tile_base + m) * 4 + quad;
       cnst[m] = group < n_groups_real ? __ldg(tok_const + int64_t(m_tile_base + m) * kTileM + quad * 32 + lane) : 0;
     }
-    uint32_t tile_seq = 0;
-    int last_u = -1;
-    TileIter it;
-    it.u = blockIdx.x;
-    it.load(unit_start, unit_end, n_units);
-    auto flush_all = [&]() {
+    const auto flush_all = [&]() {
 #pragma unroll
       for (int m = 0; m < NM; ++m) {
         const int group = (m_tile_base + m) * 4 + quad;
-        if (group < n_groups_real && cur_page[m] >= 0) {
-          const int s = warp_sum(runmax[m] + cnst[m]);
-          if (lane == 0) group_scores[int64_t(group) * ld + cur_page[m]] = s;
-        }
+        runs[m].flush([&](int page, int rm) { store(group, cnst[m], page, rm); });
       }
     };
-#pragma unroll
-    for (int m = 0; m < NM; ++m) cur_page[m] = -1;
-    for (; it.valid(n_units); it.next(unit_start, unit_end, n_units), ++tile_seq) {
+    uint32_t tile_seq = 0;
+    int last_u = -1;
+    UnitWalk it;
+    for (it.init(blockIdx.x, gridDim.x, unit_start, unit_end, n_units); it.valid(n_units);
+         it.next(unit_start, unit_end, n_units), ++tile_seq) {
       if (it.u != last_u) {  // new unit: units end on page boundaries
-        if (last_u >= 0) flush_all();
-#pragma unroll
-        for (int m = 0; m < NM; ++m) cur_page[m] = -1;
+        flush_all();
         last_u = it.u;
       }
-      const int cb = it.c0 + 4 * it.t;
       int pg[4];
-#pragma unroll
-      for (int j = 0; j < 4; ++j) pg[j] = (cb + j < it.c1) ? __ldg(chunk_page + cb + j) : -1;
+      tile_pages(chunk_page, it.chunk(), it.c1, pg);
 #pragma unroll 1
       for (int m = 0; m < NM; ++m) {
         const uint32_t seq = tile_seq * NM + m;
-        const uint32_t buf = seq & (kBAccum - 1);
+        const uint32_t buf = seq & (kNumAccum - 1);
         const int group = (m_tile_base + m) * 4 + quad;
-        int rm = 0, cp = -1, cn = 0;
+        PageRun<int> run;
+        run.rm = 0;
+        int cn = 0;
 #pragma unroll
         for (int j = 0; j < NM; ++j)
           if (j == m) {
-            rm = runmax[j];
-            cp = cur_page[j];
+            run = runs[j];
             cn = cnst[j];
           }
-        mbar_wait(&tfull[buf], (seq >> 2) & 1);
+        const auto release = [&] { mbar_arrive(&sm.tempty[buf]); };
+        mbar_wait(&sm.tfull[buf], (seq >> 2) & 1);
         tc_fence_after();
         if (group < n_groups_real) {
-          const uint32_t taddr = lane_base + buf * kTileN;
-          uint32_t va[32], vb[32];
           int cm[4];
-          tmem_ld_32x32(taddr, va);
-          tmem_ld_32x32(taddr + 32, vb);
-          tmem_ld_wait();
-          cm[0] = chunk_max_i(va);
-          cm[1] = chunk_max_i(vb);
-          tmem_ld_32x32(taddr + 64, va);
-          tmem_ld_32x32(taddr + 96, vb);
-          tmem_ld_wait();
-          tc_fence_before();
-          __syncwarp();
-          if (lane == 0) mbar_arrive(&tempty[buf]);
-          cm[2] = chunk_max_i(va);
-          cm[3] = chunk_max_i(vb);
-#pragma unroll
-          for (int j = 0; j < 4; ++j) {
-            if (pg[j] < 0) continue;
-            if (pg[j] != cp) {
-              if (cp >= 0) {
-                const int s = warp_sum(rm + cn);
-                if (lane == 0) group_scores[int64_t(group) * ld + cp] = s;
-              }
-              cp = pg[j];
-              rm = cm[j];
-            } else {
-              rm = max(rm, cm[j]);
-            }
-          }
+          drain_accum(lane_base + buf * kTileN, cm, release);
+          run.fold(pg, cm, [&](int page, int rm) { store(group, cn, page, rm); });
         } else {
-          tc_fence_before();
-          __syncwarp();
-          if (lane == 0) mbar_arrive(&tempty[buf]);
+          release_accum(release);
         }
 #pragma unroll
         for (int j = 0; j < NM; ++j)
-          if (j == m) {
-            runmax[j] = rm;
-            cur_page[j] = cp;
-          }
+          if (j == m) runs[j] = run;
       }
     }
-    if (last_u >= 0) flush_all();
-    }
+    flush_all();
   }
-
-  tc_fence_before();
-  __syncthreads();
-  if (warp == 2) {
-    tc_fence_after();
-    tmem_dealloc_512(tmem_base);
-  }
+  tile_teardown<false>(warp, tmem_base);
 }
 
-template <int NM, bool SPLIT4>
+template <int NM>
 static int launch_b1_umma_one(b200ms_t* h, const CUtensorMap& tq, const int32_t* tok_const, int m_tile_base,
                               int n_groups_real, void* scores, int64_t ld, cudaStream_t s) {
   const Corpus& c = h->corpus;
-  const uint32_t avail = kBSmemLimit - 1024 - 2048 - NM * kBTileBytes;
-  int stages = int(avail / kBTileBytes);
-  if (stages > 8) stages = 8;
-  const uint32_t smem = 1024 + NM * kBTileBytes + uint32_t(stages) * kBTileBytes + 2048;
-  auto kern = maxsim_b1_umma_kernel<NM, SPLIT4>;
-  if (int e = ensure_smem(h, reinterpret_cast<const void*>(kern), int(smem), "cudaFuncSetAttribute(maxsim_b1_umma)"))
-    return e;
-  int grid = h->max_ctas > 0 ? h->max_ctas : h->num_sms;
-  if (grid > c.n_units) grid = c.n_units;
-  if (grid < 1) return B200MS_OK;
   const int32_t* us = static_cast<const int32_t*>(h->unit_start.p);
-  kern<<<grid, kBThreads, smem, s>>>(static_cast<const uint4*>(c.rows), c.n_rows, tq, tok_const,
-                                    static_cast<const int32_t*>(h->chunk_page.p), us, us + 1, c.n_units, m_tile_base,
-                                    n_groups_real, static_cast<int32_t*>(scores), ld, stages);
-  h->launches++;
-  return check_cuda(h, cudaGetLastError(), "launch maxsim_b1_umma");
+  return launch_persistent(h, maxsim_b1_umma_kernel<NM>, "maxsim_b1_umma", kBThreads, NM * kSubtileBytes, kSubtileBytes, 8,
+                           c.n_units, s, static_cast<const uint4*>(c.rows), c.n_rows, tq, tok_const,
+                           static_cast<const int32_t*>(h->chunk_page.p), us, us + 1, c.n_units, m_tile_base, n_groups_real,
+                           static_cast<int32_t*>(scores), ld);
 }
 
 int launch_score_b1_umma(b200ms_t* h, const void* q_bits, const int32_t* group_ntok_dev, int n_groups_real,
@@ -441,12 +255,7 @@ int launch_score_b1_umma(b200ms_t* h, const void* q_bits, const int32_t* group_n
   h->launches++;
   if (int e = check_cuda(h, cudaGetLastError(), "launch b1_query_expand")) return e;
   const int n_mtiles = n_groups_padded / 4;
-  if (n_groups_real == 1) {  // single 32-token group: replicated-query form, 32-row TMA boxes
-    h->tmap_q_base = nullptr;  // this path re-encodes the shared descriptor with its own box shape
-    if (int e = make_tmap_rows(h, &h->tmap_q, q_i8, B200MS_I8, n_rows, 32)) return e;
-    return launch_b1_umma_one<1, true>(h, h->tmap_q, tok_const, 0, n_groups_real, group_scores, ld, s);
-  }
-  h->tmap_q_base = nullptr;
+  h->tmap_q_base = nullptr;  // tmap_q now describes q_i8: the next bf16 / int8 / fp8 scan must re-encode it
   if (int e = make_tmap_rows(h, &h->tmap_q, q_i8, B200MS_I8, n_rows, kTileM)) return e;
   for (int base = 0; base < n_mtiles;) {
     const int rem = n_mtiles - base;
@@ -454,9 +263,9 @@ int launch_score_b1_umma(b200ms_t* h, const void* q_bits, const int32_t* group_n
     while (nm < rem && nm < 4) nm <<= 1;
     int e;
     switch (nm) {
-      case 1: e = launch_b1_umma_one<1, false>(h, h->tmap_q, tok_const, base, n_groups_real, group_scores, ld, s); break;
-      case 2: e = launch_b1_umma_one<2, false>(h, h->tmap_q, tok_const, base, n_groups_real, group_scores, ld, s); break;
-      default: e = launch_b1_umma_one<4, false>(h, h->tmap_q, tok_const, base, n_groups_real, group_scores, ld, s); break;
+      case 1: e = launch_b1_umma_one<1>(h, h->tmap_q, tok_const, base, n_groups_real, group_scores, ld, s); break;
+      case 2: e = launch_b1_umma_one<2>(h, h->tmap_q, tok_const, base, n_groups_real, group_scores, ld, s); break;
+      default: e = launch_b1_umma_one<4>(h, h->tmap_q, tok_const, base, n_groups_real, group_scores, ld, s); break;
     }
     if (e) return e;
     base += nm;

@@ -36,6 +36,43 @@ namespace bms {
 
 constexpr int kThreads = 384;
 
+// TMA producer (one thread): the NM resident query tiles once, then every patch tile of this CTA's units through the
+// num_stages ring.
+template <int KIND, int NM>
+__device__ __forceinline__ void produce_tiles(const CUtensorMap* tmap_rows, const CUtensorMap* tmap_q, const TileSmem& sm,
+                                              int num_stages, const int32_t* __restrict__ unit_start,
+                                              const int32_t* __restrict__ unit_end, int n_units, int m_tile_base) {
+  using K = Kind<KIND>;
+  const uint64_t pol_rows = policy_evict_first();
+  const uint64_t pol_q = policy_evict_last();
+  mbar_expect_tx(sm.qfull, NM * K::kTileBytes);
+#pragma unroll
+  for (int m = 0; m < NM; ++m)
+#pragma unroll
+    for (int p = 0; p < K::kPanels; ++p)
+      tma_load_2d(tmap_q, sm.qfull, sm.q + m * K::kTileBytes + p * kSubtileBytes, p * K::kPanelElems,
+                  (m_tile_base + m) * kTileM, pol_q);
+  int stage = 0;
+  uint32_t phase = 0;
+  for (int u = blockIdx.x; u < n_units; u += gridDim.x) {
+    const int c0 = __ldg(unit_start + u), c1 = __ldg(unit_end + u);
+    const int n_tiles = (c1 - c0 + 3) >> 2;
+    for (int t = 0; t < n_tiles; ++t) {
+      mbar_wait(&sm.empty[stage], phase ^ 1);
+      mbar_expect_tx(&sm.full[stage], K::kTileBytes);
+      uint8_t* dst = sm.st + size_t(stage) * K::kTileBytes;
+      const int row0 = (c0 + 4 * t) * kGroup;
+#pragma unroll
+      for (int p = 0; p < K::kPanels; ++p)
+        tma_load_2d(tmap_rows, &sm.full[stage], dst + p * kSubtileBytes, p * K::kPanelElems, row0, pol_rows);
+      if (++stage == num_stages) {
+        stage = 0;
+        phase ^= 1;
+      }
+    }
+  }
+}
+
 // One CTA per SM, NM = 1 or 2 resident query tiles, two epilogue warpgroups (warpgroup e owns query tiles m == e mod 2;
 // at NM = 1 only warpgroup 0 works).  The lone-query / rerank kernel: HBM-bound while NM * 128 <= ~256 query tokens.
 template <int KIND, int NM>
@@ -48,86 +85,26 @@ maxsim_umma_kernel(const __grid_constant__ CUtensorMap tmap_rows, const __grid_c
   using K = Kind<KIND>;
   using Acc = typename K::Acc;
   static_assert(NM == 1 || NM == 2, "two-warpgroup form: 1 or 2 query tiles (4 and 8 run on maxsim_umma_w4_kernel)");
-  constexpr int NWG = NM;                      // epilogue warpgroups in use
-  constexpr int kKSteps = K::kKSteps;          // tcgen05.mma K steps per tile (32 B of K each)
 
   extern __shared__ uint8_t smem_raw[];
-  uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
-  uint8_t* smem_q = smem;                                            // NM query tiles
-  uint8_t* smem_st = smem + NM * K::kTileBytes;                      // num_stages patch tiles
-  uint64_t* bars = reinterpret_cast<uint64_t*>(smem_st + size_t(num_stages) * K::kTileBytes);
-  uint64_t* full = bars;                     // [num_stages] TMA -> MMA
-  uint64_t* empty = bars + 16;               // [num_stages] MMA -> TMA
-  uint64_t* tfull = bars + 32;               // [kNumAccum]  MMA -> epilogue
-  uint64_t* tempty = bars + 40;              // [kNumAccum]  epilogue -> MMA
-  uint64_t* qfull = bars + 48;               // query tiles landed
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + 56);
-
+  const TileSmem sm = carve_tile_smem(smem_raw, NM * K::kTileBytes, K::kTileBytes, num_stages);
   const int warp = threadIdx.x >> 5;
   const int lane = threadIdx.x & 31;
-
-  if (warp == 0 && lane == 0) {
-    prefetch_tmap(&tmap_rows);
-    prefetch_tmap(&tmap_q);
-    for (int i = 0; i < num_stages; ++i) {
-      mbar_init(&full[i], 1);
-      mbar_init(&empty[i], 1);
-    }
-    for (int i = 0; i < kNumAccum; ++i) {
-      mbar_init(&tfull[i], 1);
-      mbar_init(&tempty[i], 4);  // one arrive per epilogue warp of the owning warpgroup
-    }
-    mbar_init(qfull, 1);
-    fence_mbar_init();
-  }
-  if (warp == 2) tmem_alloc_512(tmem_slot);
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  const uint32_t tmem_base = *tmem_slot;
+  // tempty: one arrive per epilogue warp of the owning warpgroup
+  const uint32_t tmem_base = tile_prologue<false>(sm, warp, &tmap_rows, &tmap_q, num_stages, 1, kNumAccum, 4);
 
   if (warp == 0) {
-    // ================================================================ TMA producer
-    if (lane == 0) {
-      const uint64_t pol_rows = policy_evict_first();
-      const uint64_t pol_q = policy_evict_last();
-      mbar_expect_tx(qfull, NM * K::kTileBytes);
-#pragma unroll
-      for (int m = 0; m < NM; ++m)
-#pragma unroll
-        for (int p = 0; p < K::kPanels; ++p)
-          tma_load_2d(&tmap_q, qfull, smem_q + m * K::kTileBytes + p * kSubtileBytes, p * K::kPanelElems,
-                      (m_tile_base + m) * kTileM, pol_q);
-      int stage = 0;
-      uint32_t phase = 0;
-      for (int u = blockIdx.x; u < n_units; u += gridDim.x) {
-        const int c0 = __ldg(unit_start + u), c1 = __ldg(unit_end + u);
-        const int n_tiles = (c1 - c0 + 3) >> 2;
-        for (int t = 0; t < n_tiles; ++t) {
-          mbar_wait(&empty[stage], phase ^ 1);
-          mbar_expect_tx(&full[stage], K::kTileBytes);
-          uint8_t* dst = smem_st + size_t(stage) * K::kTileBytes;
-          const int row0 = (c0 + 4 * t) * kGroup;
-#pragma unroll
-          for (int p = 0; p < K::kPanels; ++p)
-            tma_load_2d(&tmap_rows, &full[stage], dst + p * kSubtileBytes, p * K::kPanelElems, row0, pol_rows);
-          if (++stage == num_stages) {
-            stage = 0;
-            phase ^= 1;
-          }
-        }
-      }
-    }
+    if (lane == 0) produce_tiles<KIND, NM>(&tmap_rows, &tmap_q, sm, num_stages, unit_start, unit_end, n_units, m_tile_base);
   } else if (warp == 1) {
     // ================================================================ MMA issuer
     // The whole warp walks the loop (so every address/descriptor is warp-uniform and lives in uniform registers);
     // only the tcgen05.mma / tcgen05.commit themselves are issued by the lane elect.sync picks.
     constexpr uint32_t idesc = umma_idesc(KIND, kTileM, kTileN);
     constexpr uint32_t kTileDesc = K::kTileBytes >> 4;  // tile size in descriptor units (16 B)
-    mbar_wait(qfull, 0);
+    mbar_wait(sm.qfull, 0);
     tc_fence_after();
-    const uint64_t a_desc0 = umma_desc_kmajor_sw128(smem_u32(smem_q));
-    const uint64_t b_desc0 = umma_desc_kmajor_sw128(smem_u32(smem_st));
+    const uint64_t a_desc0 = umma_desc_kmajor_sw128(smem_u32(sm.q));
+    const uint64_t b_desc0 = umma_desc_kmajor_sw128(smem_u32(sm.st));
     int stage = 0;
     uint32_t phase = 0;
     uint32_t seq = 0;
@@ -135,27 +112,21 @@ maxsim_umma_kernel(const __grid_constant__ CUtensorMap tmap_rows, const __grid_c
       const int c0 = __ldg(unit_start + u), c1 = __ldg(unit_end + u);
       const int n_tiles = (c1 - c0 + 3) >> 2;
       for (int t = 0; t < n_tiles; ++t) {
-        mbar_wait(&full[stage], phase);
+        mbar_wait(&sm.full[stage], phase);
         tc_fence_after();
         const uint64_t bd = b_desc0 + uint64_t(uint32_t(stage) * kTileDesc);
 #pragma unroll 1
         for (int m = 0; m < NM; ++m, ++seq) {
           const uint32_t buf = seq & (kNumAccum - 1);
-          mbar_wait(&tempty[buf], ((seq >> 2) & 1) ^ 1);
+          mbar_wait(&sm.tempty[buf], ((seq >> 2) & 1) ^ 1);
           tc_fence_after();
           if (elect_one()) {
-            const uint32_t d_tmem = tmem_base + buf * kTileN;
-            const uint64_t ad = a_desc0 + uint64_t(uint32_t(m) * kTileDesc);
-#pragma unroll
-            for (int ks = 0; ks < kKSteps; ++ks) {  // 32 B of K per step; 4 steps per 128 B panel
-              const uint32_t off = ((ks >> 2) * kSubtileBytes + (ks & 3) * 32) >> 4;
-              umma_ss<KIND>(d_tmem, ad + off, bd + off, idesc, ks != 0);
-            }
-            umma_commit(&tfull[buf]);
+            umma_tile<KIND>(tmem_base + buf * kTileN, a_desc0 + uint64_t(uint32_t(m) * kTileDesc), bd, idesc);
+            umma_commit(&sm.tfull[buf]);
           }
           __syncwarp();
         }
-        if (elect_one()) umma_commit(&empty[stage]);  // stage reusable once every query tile has consumed it
+        if (elect_one()) umma_commit(&sm.empty[stage]);  // stage reusable once every query tile has consumed it
         __syncwarp();
         if (++stage == num_stages) {
           stage = 0;
@@ -168,80 +139,39 @@ maxsim_umma_kernel(const __grid_constant__ CUtensorMap tmap_rows, const __grid_c
     const int wg = (warp - 4) >> 2;
     const int quad = warp & 3;  // TMEM lane quadrant this warp may access
     const uint32_t lane_base = tmem_base + (uint32_t(quad * 32) << 16);
-    if (wg < NWG) {
+    if (wg < NM) {
       const int m = wg;  // the query tile this warpgroup owns
       const int group = (m_tile_base + m) * 4 + quad;
       const bool active = group < n_groups_real;
-      Acc rm = Acc(0);
-      int cp = -1;
+      PageRun<Acc> run;
       uint32_t tile_seq = 0;
       for (int u = blockIdx.x; u < n_units; u += gridDim.x) {
         const int c0 = __ldg(unit_start + u), c1 = __ldg(unit_end + u);
         const int n_tiles = (c1 - c0 + 3) >> 2;
-        cp = -1;
+        const auto emit = [&](int page, Acc rm) {
+          store_group_score(group_scores, ld, group, slot_mode ? u : page, clamp_bits, rm);
+        };
         for (int t = 0; t < n_tiles; ++t, ++tile_seq) {
-          const int cb = c0 + 4 * t;
           int pg[4];
-#pragma unroll
-          for (int j = 0; j < 4; ++j) pg[j] = (cb + j < c1) ? __ldg(chunk_page + cb + j) : -1;
+          tile_pages(chunk_page, c0 + 4 * t, c1, pg);
           const uint32_t seq = tile_seq * NM + m;
           const uint32_t buf = seq & (kNumAccum - 1);
-          mbar_wait(&tfull[buf], (seq >> 2) & 1);
+          const auto release = [&] { mbar_arrive(&sm.tempty[buf]); };  // accumulator drained: MMA may overwrite it
+          mbar_wait(&sm.tfull[buf], (seq >> 2) & 1);
           tc_fence_after();
           if (active) {
-            const uint32_t taddr = lane_base + buf * kTileN;
             Acc cm[4];
-            uint32_t va[32], vb[32];
-            tmem_ld_32x32(taddr, va);
-            tmem_ld_32x32(taddr + 32, vb);
-            tmem_ld_wait();
-            cm[0] = chunk_max<Acc>(va);
-            cm[1] = chunk_max<Acc>(vb);
-            tmem_ld_32x32(taddr + 64, va);
-            tmem_ld_32x32(taddr + 96, vb);
-            tmem_ld_wait();
-            tc_fence_before();
-            __syncwarp();
-            if (lane == 0) mbar_arrive(&tempty[buf]);  // accumulator drained: MMA may overwrite it
-            cm[2] = chunk_max<Acc>(va);
-            cm[3] = chunk_max<Acc>(vb);
-#pragma unroll
-            for (int j = 0; j < 4; ++j) {
-              if (pg[j] < 0) continue;  // chunk belongs to the next unit
-              if (pg[j] != cp) {
-                if (cp >= 0) {
-                  const int o = slot_mode ? u : cp;
-                  const Acc s = warp_sum(clamp_token_max(clamp_bits, o, rm));
-                  if (lane == 0) group_scores[int64_t(group) * ld + o] = s;
-                }
-                cp = pg[j];
-                rm = cm[j];
-              } else {
-                rm = acc_max(rm, cm[j]);
-              }
-            }
+            drain_accum(lane_base + buf * kTileN, cm, release);
+            run.fold(pg, cm, emit);
           } else {
-            tc_fence_before();
-            __syncwarp();
-            if (lane == 0) mbar_arrive(&tempty[buf]);
+            release_accum(release);
           }
         }
-        // unit ends on a page boundary: flush the open page
-        if (active && cp >= 0) {
-          const int o = slot_mode ? u : cp;
-          const Acc s = warp_sum(clamp_token_max(clamp_bits, o, rm));
-          if (lane == 0) group_scores[int64_t(group) * ld + o] = s;
-        }
+        run.flush(emit);  // units end on a page boundary
       }
     }
   }
-
-  tc_fence_before();
-  __syncthreads();
-  if (warp == 2) {
-    tc_fence_after();
-    tmem_dealloc_512(tmem_base);
-  }
+  tile_teardown<false>(warp, tmem_base);
 }
 
 // ================================================================================================================
@@ -262,81 +192,22 @@ maxsim_umma_w4_kernel(const __grid_constant__ CUtensorMap tmap_rows, const __gri
   using Acc = typename K::Acc;
   static_assert(NM % 4 == 0, "W4 form needs a multiple of four query tiles");
   constexpr int MPW = NM / 4;                  // query tiles per epilogue warpgroup
-  constexpr int kKSteps = K::kKSteps;
 
   extern __shared__ uint8_t smem_raw[];
-  uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
-  uint8_t* smem_q = smem;
-  uint8_t* smem_st = smem + NM * K::kTileBytes;
-  uint64_t* bars = reinterpret_cast<uint64_t*>(smem_st + size_t(num_stages) * K::kTileBytes);
-  uint64_t* full = bars;
-  uint64_t* empty = bars + 16;
-  uint64_t* tfull = bars + 32;
-  uint64_t* tempty = bars + 40;
-  uint64_t* qfull = bars + 48;
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + 56);
-
+  const TileSmem sm = carve_tile_smem(smem_raw, NM * K::kTileBytes, K::kTileBytes, num_stages);
   const int warp = threadIdx.x >> 5;
   const int lane = threadIdx.x & 31;
-
-  if (warp == 0 && lane == 0) {
-    prefetch_tmap(&tmap_rows);
-    prefetch_tmap(&tmap_q);
-    for (int i = 0; i < num_stages; ++i) {
-      mbar_init(&full[i], 1);
-      mbar_init(&empty[i], 1);
-    }
-    for (int i = 0; i < kNumAccum; ++i) {
-      mbar_init(&tfull[i], 1);
-      mbar_init(&tempty[i], 4);
-    }
-    mbar_init(qfull, 1);
-    fence_mbar_init();
-  }
-  if (warp == 2) tmem_alloc_512(tmem_slot);
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  const uint32_t tmem_base = *tmem_slot;
+  const uint32_t tmem_base = tile_prologue<false>(sm, warp, &tmap_rows, &tmap_q, num_stages, 1, kNumAccum, 4);
 
   if (warp == 0) {
-    if (lane == 0) {
-      const uint64_t pol_rows = policy_evict_first();
-      const uint64_t pol_q = policy_evict_last();
-      mbar_expect_tx(qfull, NM * K::kTileBytes);
-#pragma unroll
-      for (int m = 0; m < NM; ++m)
-#pragma unroll
-        for (int p = 0; p < K::kPanels; ++p)
-          tma_load_2d(&tmap_q, qfull, smem_q + m * K::kTileBytes + p * kSubtileBytes, p * K::kPanelElems,
-                      (m_tile_base + m) * kTileM, pol_q);
-      int stage = 0;
-      uint32_t phase = 0;
-      for (int u = blockIdx.x; u < n_units; u += gridDim.x) {
-        const int c0 = __ldg(unit_start + u), c1 = __ldg(unit_end + u);
-        const int n_tiles = (c1 - c0 + 3) >> 2;
-        for (int t = 0; t < n_tiles; ++t) {
-          mbar_wait(&empty[stage], phase ^ 1);
-          mbar_expect_tx(&full[stage], K::kTileBytes);
-          uint8_t* dst = smem_st + size_t(stage) * K::kTileBytes;
-          const int row0 = (c0 + 4 * t) * kGroup;
-#pragma unroll
-          for (int p = 0; p < K::kPanels; ++p)
-            tma_load_2d(&tmap_rows, &full[stage], dst + p * kSubtileBytes, p * K::kPanelElems, row0, pol_rows);
-          if (++stage == num_stages) {
-            stage = 0;
-            phase ^= 1;
-          }
-        }
-      }
-    }
+    if (lane == 0) produce_tiles<KIND, NM>(&tmap_rows, &tmap_q, sm, num_stages, unit_start, unit_end, n_units, m_tile_base);
   } else if (warp == 1) {
     constexpr uint32_t idesc = umma_idesc(KIND, kTileM, kTileN);
     constexpr uint32_t kTileDesc = K::kTileBytes >> 4;
-    mbar_wait(qfull, 0);
+    mbar_wait(sm.qfull, 0);
     tc_fence_after();
-    const uint64_t a_desc0 = umma_desc_kmajor_sw128(smem_u32(smem_q));
-    const uint64_t b_desc0 = umma_desc_kmajor_sw128(smem_u32(smem_st));
+    const uint64_t a_desc0 = umma_desc_kmajor_sw128(smem_u32(sm.q));
+    const uint64_t b_desc0 = umma_desc_kmajor_sw128(smem_u32(sm.st));
     int stage = 0;
     uint32_t phase = 0;
     uint32_t use = 0;  // uses of every accumulator so far (each tile uses each buffer MPW times)
@@ -344,29 +215,23 @@ maxsim_umma_w4_kernel(const __grid_constant__ CUtensorMap tmap_rows, const __gri
       const int c0 = __ldg(unit_start + u), c1 = __ldg(unit_end + u);
       const int n_tiles = (c1 - c0 + 3) >> 2;
       for (int t = 0; t < n_tiles; ++t) {
-        mbar_wait(&full[stage], phase);
+        mbar_wait(&sm.full[stage], phase);
         tc_fence_after();
         const uint64_t bd = b_desc0 + uint64_t(uint32_t(stage) * kTileDesc);
 #pragma unroll 1
         for (int m = 0; m < NM; ++m) {
           const uint32_t buf = m & 3;
           const uint32_t n = use + (m >> 2);
-          mbar_wait(&tempty[buf], (n & 1) ^ 1);
+          mbar_wait(&sm.tempty[buf], (n & 1) ^ 1);
           tc_fence_after();
           if (elect_one()) {
-            const uint32_t d_tmem = tmem_base + buf * kTileN;
-            const uint64_t ad = a_desc0 + uint64_t(uint32_t(m) * kTileDesc);
-#pragma unroll
-            for (int ks = 0; ks < kKSteps; ++ks) {
-              const uint32_t off = ((ks >> 2) * kSubtileBytes + (ks & 3) * 32) >> 4;
-              umma_ss<KIND>(d_tmem, ad + off, bd + off, idesc, ks != 0);
-            }
-            umma_commit(&tfull[buf]);
+            umma_tile<KIND>(tmem_base + buf * kTileN, a_desc0 + uint64_t(uint32_t(m) * kTileDesc), bd, idesc);
+            umma_commit(&sm.tfull[buf]);
           }
           __syncwarp();
         }
         use += MPW;
-        if (elect_one()) umma_commit(&empty[stage]);
+        if (elect_one()) umma_commit(&sm.empty[stage]);
         __syncwarp();
         if (++stage == num_stages) {
           stage = 0;
@@ -378,127 +243,58 @@ maxsim_umma_w4_kernel(const __grid_constant__ CUtensorMap tmap_rows, const __gri
     const int wg = (warp - 4) >> 2;  // 0..3 = accumulator buffer owned
     const int quad = warp & 3;
     const uint32_t taddr = tmem_base + (uint32_t(quad * 32) << 16) + wg * kTileN;
-    Acc runmax[MPW];
-    int cur_page[MPW];
+    const auto release = [&] { mbar_arrive(&sm.tempty[wg]); };
+    PageRun<Acc> run[MPW];
     uint32_t use = 0;
     for (int u = blockIdx.x; u < n_units; u += gridDim.x) {
       const int c0 = __ldg(unit_start + u), c1 = __ldg(unit_end + u);
       const int n_tiles = (c1 - c0 + 3) >> 2;
-#pragma unroll
-      for (int i = 0; i < MPW; ++i) cur_page[i] = -1;
       for (int t = 0; t < n_tiles; ++t) {
-        const int cb = c0 + 4 * t;
         int pg[4];
-#pragma unroll
-        for (int j = 0; j < 4; ++j) pg[j] = (cb + j < c1) ? __ldg(chunk_page + cb + j) : -1;
+        tile_pages(chunk_page, c0 + 4 * t, c1, pg);
 #pragma unroll
         for (int i = 0; i < MPW; ++i, ++use) {
-          const int m = wg + 4 * i;
-          const int group = (m_tile_base + m) * 4 + quad;
-          mbar_wait(&tfull[wg], use & 1);
+          const int group = (m_tile_base + wg + 4 * i) * 4 + quad;
+          mbar_wait(&sm.tfull[wg], use & 1);
           tc_fence_after();
           if (group < n_groups_real) {
-            uint32_t va[32], vb[32];
             Acc cm[4];
-            tmem_ld_32x32(taddr, va);
-            tmem_ld_32x32(taddr + 32, vb);
-            tmem_ld_wait();
-            cm[0] = chunk_max<Acc>(va);
-            cm[1] = chunk_max<Acc>(vb);
-            tmem_ld_32x32(taddr + 64, va);
-            tmem_ld_32x32(taddr + 96, vb);
-            tmem_ld_wait();
-            tc_fence_before();
-            __syncwarp();
-            if (lane == 0) mbar_arrive(&tempty[wg]);
-            cm[2] = chunk_max<Acc>(va);
-            cm[3] = chunk_max<Acc>(vb);
-#pragma unroll
-            for (int j = 0; j < 4; ++j) {
-              if (pg[j] < 0) continue;
-              if (pg[j] != cur_page[i]) {
-                if (cur_page[i] >= 0) {
-                  const int o = slot_mode ? u : cur_page[i];
-                  const Acc s2 = warp_sum(clamp_token_max(clamp_bits, o, runmax[i]));
-                  if (lane == 0) group_scores[int64_t(group) * ld + o] = s2;
-                }
-                cur_page[i] = pg[j];
-                runmax[i] = cm[j];
-              } else {
-                runmax[i] = acc_max(runmax[i], cm[j]);
-              }
-            }
+            drain_accum(taddr, cm, release);
+            run[i].fold(pg, cm, [&](int page, Acc rm) {
+              store_group_score(group_scores, ld, group, slot_mode ? u : page, clamp_bits, rm);
+            });
           } else {
-            tc_fence_before();
-            __syncwarp();
-            if (lane == 0) mbar_arrive(&tempty[wg]);
+            release_accum(release);
           }
         }
       }
 #pragma unroll
       for (int i = 0; i < MPW; ++i) {
         const int group = (m_tile_base + wg + 4 * i) * 4 + quad;
-        if (group < n_groups_real && cur_page[i] >= 0) {
-          const int o = slot_mode ? u : cur_page[i];
-          const Acc s2 = warp_sum(clamp_token_max(clamp_bits, o, runmax[i]));
-          if (lane == 0) group_scores[int64_t(group) * ld + o] = s2;
-        }
+        run[i].flush([&](int page, Acc rm) {
+          store_group_score(group_scores, ld, group, slot_mode ? u : page, clamp_bits, rm);
+        });
       }
     }
   }
-
-  tc_fence_before();
-  __syncthreads();
-  if (warp == 2) {
-    tc_fence_after();
-    tmem_dealloc_512(tmem_base);
-  }
-}
-
-template <int KIND, int NM>
-static int launch_w4(b200ms_t* h, const UnitPlan& up, const CUtensorMap& tq, int m_tile_base, int n_groups_real,
-                     void* scores, int64_t ld, cudaStream_t s) {
-  using K = Kind<KIND>;
-  const Corpus& c = h->corpus;
-  const uint32_t avail = kSmemLimit - 1024 - kBarrierBytes - NM * K::kTileBytes;
-  int stages = int(avail / K::kTileBytes);
-  if (stages > 8) stages = 8;
-  if (stages < 2) return set_error(h, B200MS_EINVAL, "maxsim_umma_w4: not enough shared memory for 2 stages");
-  const uint32_t smem = 1024 + NM * K::kTileBytes + uint32_t(stages) * K::kTileBytes + kBarrierBytes;
-  auto kern = maxsim_umma_w4_kernel<KIND, NM>;
-  if (int e = ensure_smem(h, reinterpret_cast<const void*>(kern), int(smem), "cudaFuncSetAttribute(maxsim_umma_w4)"))
-    return e;
-  int grid = h->max_ctas > 0 ? h->max_ctas : h->num_sms;
-  if (grid > up.n_units) grid = up.n_units;
-  if (grid < 1) return B200MS_OK;
-  kern<<<grid, kThreadsW4, smem, s>>>(c.tmap, tq, static_cast<const int32_t*>(h->chunk_page.p), up.start, up.end, up.slot_mode,
-                                     up.n_units, m_tile_base, n_groups_real, up.clamp_bits,
-                                     static_cast<typename K::Acc*>(scores), ld, stages);
-  h->launches++;
-  return check_cuda(h, cudaGetLastError(), "launch maxsim_umma_w4");
+  tile_teardown<false>(warp, tmem_base);
 }
 
 // ---------------------------------------------------------------------------------------------- host side
+// One launch of a one-CTA form: NM = 1 / 2 on maxsim_umma_kernel with up to 14 stages (16 KB tiles: 8 stages = 128 KB in
+// flight left the one-byte scans latency-bound), NM = 4 / 8 on the W4 form with up to 8.
 template <int KIND, int NM>
 static int launch_one(b200ms_t* h, const UnitPlan& up, const CUtensorMap& tq, int m_tile_base, int n_groups_real,
                       void* scores, int64_t ld, cudaStream_t s) {
   using K = Kind<KIND>;
-  const Corpus& c = h->corpus;
-  const uint32_t avail = kSmemLimit - 1024 /*align*/ - kBarrierBytes - NM * K::kTileBytes;
-  int stages = int(avail / K::kTileBytes);
-  if (stages > 14) stages = 14;  // 16 KB tiles: 8 stages = 128 KB in flight left the one-byte scans latency-bound (full[16])
-  const uint32_t smem = 1024 + NM * K::kTileBytes + uint32_t(stages) * K::kTileBytes + kBarrierBytes;
-  auto kern = maxsim_umma_kernel<KIND, NM>;
-  if (int e = ensure_smem(h, reinterpret_cast<const void*>(kern), int(smem), "cudaFuncSetAttribute(maxsim_umma)"))
-    return e;
-  int grid = h->max_ctas > 0 ? h->max_ctas : h->num_sms;
-  if (grid > up.n_units) grid = up.n_units;
-  if (grid < 1) return B200MS_OK;
-  kern<<<grid, kThreads, smem, s>>>(c.tmap, tq, static_cast<const int32_t*>(h->chunk_page.p), up.start, up.end, up.slot_mode,
-                                   up.n_units, m_tile_base, n_groups_real, up.clamp_bits,
-                                   static_cast<typename K::Acc*>(scores), ld, stages);
-  h->launches++;
-  return check_cuda(h, cudaGetLastError(), "launch maxsim_umma");
+  const auto launch = [&](auto kern, const char* name, int threads, int max_stages) {
+    return launch_persistent(h, kern, name, threads, NM * K::kTileBytes, K::kTileBytes, max_stages, up.n_units, s,
+                             h->corpus.tmap, tq, static_cast<const int32_t*>(h->chunk_page.p), up.start, up.end,
+                             up.slot_mode, up.n_units, m_tile_base, n_groups_real, up.clamp_bits,
+                             static_cast<typename K::Acc*>(scores), ld);
+  };
+  if constexpr (NM <= 2) return launch(maxsim_umma_kernel<KIND, NM>, "maxsim_umma", kThreads, 14);
+  else return launch(maxsim_umma_w4_kernel<KIND, NM>, "maxsim_umma_w4", kThreadsW4, 8);
 }
 
 // Pass planner: score query tiles [0, n_mtiles) against the unit plan with as few passes over the corpus as possible.
@@ -534,10 +330,10 @@ static int launch_kind(b200ms_t* h, const UnitPlan& up, const CUtensorMap& tq, i
     switch (nm) {
       case 1: e = launch_one<KIND, 1>(h, up, tq, base, n_groups_real, scores, ld, s); break;
       case 2: e = launch_one<KIND, 2>(h, up, tq, base, n_groups_real, scores, ld, s); break;
-      case 4: e = launch_w4<KIND, 4>(h, up, tq, base, n_groups_real, scores, ld, s); break;
+      case 4: e = launch_one<KIND, 4>(h, up, tq, base, n_groups_real, scores, ld, s); break;
       default:
         if constexpr (kMaxNM >= 8) {
-          e = launch_w4<KIND, 8>(h, up, tq, base, n_groups_real, scores, ld, s);
+          e = launch_one<KIND, 8>(h, up, tq, base, n_groups_real, scores, ld, s);
         } else {
           e = set_error(h, B200MS_EINVAL, "maxsim_umma: bad NM");
         }

@@ -40,20 +40,9 @@ maxsim_umma_pair_kernel(const __grid_constant__ CUtensorMap tmap_rows, const __g
   using Acc = typename K::Acc;
   static_assert(NM % 2 == 0, "pair form: an even number of query tiles per CTA (tile m uses accumulator m & 1)");
   constexpr int MPW = NM / 2;  // query tiles per epilogue warpgroup
-  constexpr int kKSteps = K::kKSteps;
 
   extern __shared__ uint8_t smem_raw[];
-  uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
-  uint8_t* smem_q = smem;
-  uint8_t* smem_st = smem + NM * K::kTileBytes;
-  uint64_t* bars = reinterpret_cast<uint64_t*>(smem_st + size_t(num_stages) * K::kTileBytes);
-  uint64_t* full = bars;
-  uint64_t* empty = bars + 16;
-  uint64_t* tfull = bars + 32;
-  uint64_t* tempty = bars + 40;
-  uint64_t* qfull = bars + 48;
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + 56);
-
+  const TileSmem sm = carve_tile_smem(smem_raw, NM * K::kTileBytes, K::kTileBytes, num_stages);
   const int warp = threadIdx.x >> 5;
   const int lane = threadIdx.x & 31;
   const uint32_t rank = cluster_ctarank();           // 0 = leader (issues the MMAs), 1 = peer
@@ -69,46 +58,29 @@ maxsim_umma_pair_kernel(const __grid_constant__ CUtensorMap tmap_rows, const __g
     n_iter = max(n_iter, warp_sum(acc));
   }
 
-  if (warp == 0 && lane == 0) {
-    prefetch_tmap(&tmap_rows);
-    prefetch_tmap(&tmap_q);
-    for (int i = 0; i < num_stages; ++i) {
-      mbar_init(&full[i], 1);
-      mbar_init(&empty[i], 1);
-    }
-    for (int i = 0; i < 2; ++i) {
-      mbar_init(&tfull[i], 1);
-      mbar_init(&tempty[i], 16);  // 2 CTAs x 2 warpgroups x 4 warps
-    }
-    mbar_init(qfull, 1);
-    fence_mbar_init();
-  }
-  if (warp == 2) tmem_alloc_512_pair(tmem_slot);
-  tc_fence_before();
-  cluster_sync_all();  // barrier inits + TMEM address visible in both CTAs before any remote arrive / TMA signal
-  tc_fence_after();
-  const uint32_t tmem_base = *tmem_slot;
+  // tempty: 2 CTAs x 2 warpgroups x 4 warps
+  const uint32_t tmem_base = tile_prologue<true>(sm, warp, &tmap_rows, &tmap_q, num_stages, 1, 2, 16);
 
   if (warp == 0) {
     if (lane == 0) {
       const uint64_t pol_rows = policy_evict_first();
       const uint64_t pol_q = policy_evict_last();
-      const uint32_t full_l = mapa_rank(smem_u32(full), 0);   // the LEADER's barriers collect both CTAs' bytes
-      const uint32_t qfull_l = mapa_rank(smem_u32(qfull), 0);
-      if (rank == 0) mbar_expect_tx(qfull, 2 * NM * K::kTileBytes);
+      const uint32_t full_l = mapa_rank(smem_u32(sm.full), 0);   // the LEADER's barriers collect both CTAs' bytes
+      const uint32_t qfull_l = mapa_rank(smem_u32(sm.qfull), 0);
+      if (rank == 0) mbar_expect_tx(sm.qfull, 2 * NM * K::kTileBytes);
 #pragma unroll
       for (int m = 0; m < NM; ++m)
 #pragma unroll
         for (int p = 0; p < K::kPanels; ++p)
-          tma_load_2d_pair(&tmap_q, qfull_l, smem_q + m * K::kTileBytes + p * kSubtileBytes, p * K::kPanelElems,
+          tma_load_2d_pair(&tmap_q, qfull_l, sm.q + m * K::kTileBytes + p * kSubtileBytes, p * K::kPanelElems,
                            (m_tile_base + int(rank) * NM + m) * kTileM, pol_q);
       int stage = 0;
       uint32_t phase = 0;
       int k = 0;
       auto load_tile = [&](int row0) {
-        mbar_wait(&empty[stage], phase ^ 1);
-        if (rank == 0) mbar_expect_tx(&full[stage], 2 * K::kTileBytes);
-        uint8_t* dst = smem_st + size_t(stage) * K::kTileBytes;
+        mbar_wait(&sm.empty[stage], phase ^ 1);
+        if (rank == 0) mbar_expect_tx(&sm.full[stage], 2 * K::kTileBytes);
+        uint8_t* dst = sm.st + size_t(stage) * K::kTileBytes;
 #pragma unroll
         for (int p = 0; p < K::kPanels; ++p)
           tma_load_2d_pair(&tmap_rows, full_l + uint32_t(stage) * 8u, dst + p * kSubtileBytes, p * K::kPanelElems, row0,
@@ -126,7 +98,7 @@ maxsim_umma_pair_kernel(const __grid_constant__ CUtensorMap tmap_rows, const __g
       for (; k < n_iter; ++k) load_tile(0);  // this stream is exhausted: keep the pair in step
       // tail: the multicast commits of the last stages must land before this CTA may exit
       for (int i = 0; i < num_stages; ++i) {
-        mbar_wait(&empty[stage], phase ^ 1);
+        mbar_wait(&sm.empty[stage], phase ^ 1);
         if (++stage == num_stages) {
           stage = 0;
           phase ^= 1;
@@ -137,37 +109,31 @@ maxsim_umma_pair_kernel(const __grid_constant__ CUtensorMap tmap_rows, const __g
     if (rank == 0) {
       constexpr uint32_t idesc = umma_idesc(KIND, 2 * kTileM, kPairN);
       constexpr uint32_t kTileDesc = K::kTileBytes >> 4;
-      mbar_wait(qfull, 0);
+      mbar_wait(sm.qfull, 0);
       tc_fence_after();
-      const uint64_t a_desc0 = umma_desc_kmajor_sw128(smem_u32(smem_q));
-      const uint64_t b_desc0 = umma_desc_kmajor_sw128(smem_u32(smem_st));
+      const uint64_t a_desc0 = umma_desc_kmajor_sw128(smem_u32(sm.q));
+      const uint64_t b_desc0 = umma_desc_kmajor_sw128(smem_u32(sm.st));
       int stage = 0;
       uint32_t phase = 0;
       uint32_t use = 0;  // uses of each accumulator so far
       for (int k = 0; k < n_iter; ++k) {
-        mbar_wait(&full[stage], phase);
+        mbar_wait(&sm.full[stage], phase);
         tc_fence_after();
         const uint64_t bd = b_desc0 + uint64_t(uint32_t(stage) * kTileDesc);
 #pragma unroll 1
         for (int m = 0; m < NM; ++m) {
           const uint32_t buf = m & 1;
           const uint32_t n = use + (m >> 1);
-          mbar_wait(&tempty[buf], (n & 1) ^ 1);
+          mbar_wait(&sm.tempty[buf], (n & 1) ^ 1);
           tc_fence_after();
           if (elect_one()) {
-            const uint32_t d_tmem = tmem_base + buf * kPairN;
-            const uint64_t ad = a_desc0 + uint64_t(uint32_t(m) * kTileDesc);
-#pragma unroll
-            for (int ks = 0; ks < kKSteps; ++ks) {
-              const uint32_t off = ((ks >> 2) * kSubtileBytes + (ks & 3) * 32) >> 4;
-              umma2_ss<KIND>(d_tmem, ad + off, bd + off, idesc, ks != 0);
-            }
-            umma2_commit_mc(&tfull[buf], 3);
+            umma_tile<KIND, true>(tmem_base + buf * kPairN, a_desc0 + uint64_t(uint32_t(m) * kTileDesc), bd, idesc);
+            umma2_commit_mc(&sm.tfull[buf], 3);
           }
           __syncwarp();
         }
         use += MPW;
-        if (elect_one()) umma2_commit_mc(&empty[stage], 3);
+        if (elect_one()) umma2_commit_mc(&sm.empty[stage], 3);
         __syncwarp();
         if (++stage == num_stages) {
           stage = 0;
@@ -181,92 +147,51 @@ maxsim_umma_pair_kernel(const __grid_constant__ CUtensorMap tmap_rows, const __g
     const int half = e & 1;  // column half = unit stream
     const int quad = warp & 3;
     const uint32_t taddr = tmem_base + (uint32_t(quad * 32) << 16) + buf * kPairN + half * kTileN;
-    const uint32_t tempty_l = mapa_rank(smem_u32(&tempty[buf]), 0);
-    Acc runmax[MPW];
-    int cur_page[MPW];
+    const uint32_t tempty_l = mapa_rank(smem_u32(&sm.tempty[buf]), 0);
+    const auto release = [&] { mbar_arrive_cluster(tempty_l); };
+    PageRun<Acc> run[MPW];
     uint32_t use = 0;
     int k = 0;
     for (int u = stream0 + half; u < n_units; u += gridDim.x) {
       const int c0 = __ldg(unit_start + u), c1 = __ldg(unit_end + u);
       const int n_tiles = (c1 - c0 + 3) >> 2;
-#pragma unroll
-      for (int i = 0; i < MPW; ++i) cur_page[i] = -1;
       for (int t = 0; t < n_tiles; ++t, ++k) {
-        const int cb = c0 + 4 * t;
         int pg[4];
-#pragma unroll
-        for (int j = 0; j < 4; ++j) pg[j] = (cb + j < c1) ? __ldg(chunk_page + cb + j) : -1;
+        tile_pages(chunk_page, c0 + 4 * t, c1, pg);
 #pragma unroll
         for (int i = 0; i < MPW; ++i, ++use) {
-          const int m = buf + 2 * i;
-          const int group = (m_tile_base + int(rank) * NM + m) * 4 + quad;
-          mbar_wait(&tfull[buf], use & 1);
+          const int group = (m_tile_base + int(rank) * NM + buf + 2 * i) * 4 + quad;
+          mbar_wait(&sm.tfull[buf], use & 1);
           tc_fence_after();
           if (group < n_groups_real) {
-            uint32_t va[32], vb[32];
             Acc cm[4];
-            tmem_ld_32x32(taddr, va);
-            tmem_ld_32x32(taddr + 32, vb);
-            tmem_ld_wait();
-            cm[0] = chunk_max<Acc>(va);
-            cm[1] = chunk_max<Acc>(vb);
-            tmem_ld_32x32(taddr + 64, va);
-            tmem_ld_32x32(taddr + 96, vb);
-            tmem_ld_wait();
-            tc_fence_before();
-            __syncwarp();
-            if (lane == 0) mbar_arrive_cluster(tempty_l);
-            cm[2] = chunk_max<Acc>(va);
-            cm[3] = chunk_max<Acc>(vb);
-#pragma unroll
-            for (int j = 0; j < 4; ++j) {
-              if (pg[j] < 0) continue;
-              if (pg[j] != cur_page[i]) {
-                if (cur_page[i] >= 0) {
-                  const int o = slot_mode ? u : cur_page[i];
-                  const Acc s2 = warp_sum(clamp_token_max(clamp_bits, o, runmax[i]));
-                  if (lane == 0) group_scores[int64_t(group) * ld + o] = s2;
-                }
-                cur_page[i] = pg[j];
-                runmax[i] = cm[j];
-              } else {
-                runmax[i] = acc_max(runmax[i], cm[j]);
-              }
-            }
+            drain_accum(taddr, cm, release);
+            run[i].fold(pg, cm, [&](int page, Acc rm) {
+              store_group_score(group_scores, ld, group, slot_mode ? u : page, clamp_bits, rm);
+            });
           } else {
-            tc_fence_before();
-            __syncwarp();
-            if (lane == 0) mbar_arrive_cluster(tempty_l);
+            release_accum(release);
           }
         }
       }
 #pragma unroll
       for (int i = 0; i < MPW; ++i) {
         const int group = (m_tile_base + int(rank) * NM + buf + 2 * i) * 4 + quad;
-        if (group < n_groups_real && cur_page[i] >= 0) {
-          const int o = slot_mode ? u : cur_page[i];
-          const Acc s2 = warp_sum(clamp_token_max(clamp_bits, o, runmax[i]));
-          if (lane == 0) group_scores[int64_t(group) * ld + o] = s2;
-        }
+        run[i].flush([&](int page, Acc rm) {
+          store_group_score(group_scores, ld, group, slot_mode ? u : page, clamp_bits, rm);
+        });
       }
     }
     for (; k < n_iter; ++k) {  // dummy tiles of an exhausted stream: keep the accumulator hand-shake going
 #pragma unroll
       for (int i = 0; i < MPW; ++i, ++use) {
-        mbar_wait(&tfull[buf], use & 1);
+        mbar_wait(&sm.tfull[buf], use & 1);
         __syncwarp();
-        if (lane == 0) mbar_arrive_cluster(tempty_l);
+        if (lane == 0) release();
       }
     }
   }
-
-  __syncwarp();
-  tc_fence_before();
-  cluster_sync_all();  // nobody exits (or frees TMEM) while the partner can still touch its shared memory / TMEM
-  if (warp == 2) {
-    tc_fence_after();
-    tmem_dealloc_512_pair(tmem_base);
-  }
+  tile_teardown<true>(warp, tmem_base);
 }
 
 // ================================================================================================================
@@ -275,33 +200,6 @@ maxsim_umma_pair_kernel(const __grid_constant__ CUtensorMap tmap_rows, const __g
 // unit streams, alternating per iteration: even iterations carry a tile of its stream 2c, odd ones a tile of stream 2c+1
 // (c = blockIdx.x; a stream walks units v, v + 2*gridDim.x, ...).  Warpgroup e drains accumulator e>>1 (= iteration parity)
 // and column half e&1 (= the CTA that loaded those rows), i.e. exactly one of the pair's four streams.
-struct UnitWalk {
-  int u, stride, c0, c1, t, n_tiles;
-  __device__ __forceinline__ void load(const int32_t* us, const int32_t* ue, int n_units) {
-    n_tiles = 0;
-    while (u < n_units) {
-      c0 = __ldg(us + u);
-      c1 = __ldg(ue + u);
-      n_tiles = (c1 - c0 + 3) >> 2;
-      if (n_tiles > 0) break;
-      u += stride;
-    }
-    t = 0;
-  }
-  __device__ __forceinline__ void init(int v, int stride_, const int32_t* us, const int32_t* ue, int n_units) {
-    u = v;
-    stride = stride_;
-    load(us, ue, n_units);
-  }
-  __device__ __forceinline__ bool valid(int n_units) const { return u < n_units; }
-  __device__ __forceinline__ void next(const int32_t* us, const int32_t* ue, int n_units) {
-    if (++t == n_tiles) {
-      u += stride;
-      load(us, ue, n_units);
-    }
-  }
-};
-
 template <int KIND>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreadsPair, 1)
 maxsim_umma_pair1_kernel(const __grid_constant__ CUtensorMap tmap_rows, const __grid_constant__ CUtensorMap tmap_q,
@@ -311,20 +209,9 @@ maxsim_umma_pair1_kernel(const __grid_constant__ CUtensorMap tmap_rows, const __
                          typename Kind<KIND>::Acc* __restrict__ group_scores, int64_t ld, int num_stages) {
   using K = Kind<KIND>;
   using Acc = typename K::Acc;
-  constexpr int kKSteps = K::kKSteps;
 
   extern __shared__ uint8_t smem_raw[];
-  uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
-  uint8_t* smem_q = smem;
-  uint8_t* smem_st = smem + K::kTileBytes;
-  uint64_t* bars = reinterpret_cast<uint64_t*>(smem_st + size_t(num_stages) * K::kTileBytes);
-  uint64_t* full = bars;
-  uint64_t* empty = bars + 16;
-  uint64_t* tfull = bars + 32;
-  uint64_t* tempty = bars + 40;
-  uint64_t* qfull = bars + 48;
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + 56);
-
+  const TileSmem sm = carve_tile_smem(smem_raw, K::kTileBytes, K::kTileBytes, num_stages);
   const int warp = threadIdx.x >> 5;
   const int lane = threadIdx.x & 31;
   const uint32_t rank = cluster_ctarank();
@@ -342,36 +229,18 @@ maxsim_umma_pair1_kernel(const __grid_constant__ CUtensorMap tmap_rows, const __
   }
   const int n_iter = 2 * n_half;
 
-  if (warp == 0 && lane == 0) {
-    prefetch_tmap(&tmap_rows);
-    prefetch_tmap(&tmap_q);
-    for (int i = 0; i < num_stages; ++i) {
-      mbar_init(&full[i], 1);
-      mbar_init(&empty[i], 1);
-    }
-    for (int i = 0; i < 2; ++i) {
-      mbar_init(&tfull[i], 1);
-      mbar_init(&tempty[i], 16);
-    }
-    mbar_init(qfull, 1);
-    fence_mbar_init();
-  }
-  if (warp == 2) tmem_alloc_512_pair(tmem_slot);
-  tc_fence_before();
-  cluster_sync_all();
-  tc_fence_after();
-  const uint32_t tmem_base = *tmem_slot;
+  const uint32_t tmem_base = tile_prologue<true>(sm, warp, &tmap_rows, &tmap_q, num_stages, 1, 2, 16);
 
   if (warp == 0) {
     if (lane == 0) {
       const uint64_t pol_rows = policy_evict_first();
       const uint64_t pol_q = policy_evict_last();
-      const uint32_t full_l = mapa_rank(smem_u32(full), 0);
-      const uint32_t qfull_l = mapa_rank(smem_u32(qfull), 0);
-      if (rank == 0) mbar_expect_tx(qfull, 2 * K::kTileBytes);
+      const uint32_t full_l = mapa_rank(smem_u32(sm.full), 0);
+      const uint32_t qfull_l = mapa_rank(smem_u32(sm.qfull), 0);
+      if (rank == 0) mbar_expect_tx(sm.qfull, 2 * K::kTileBytes);
 #pragma unroll
       for (int p = 0; p < K::kPanels; ++p)
-        tma_load_2d_pair(&tmap_q, qfull_l, smem_q + p * kSubtileBytes, p * K::kPanelElems,
+        tma_load_2d_pair(&tmap_q, qfull_l, sm.q + p * kSubtileBytes, p * K::kPanelElems,
                          (m_tile_base + int(rank)) * kTileM, pol_q);
       UnitWalk w0, w1;
       w0.init(2 * int(blockIdx.x), vstride, unit_start, unit_end, n_units);
@@ -382,16 +251,16 @@ maxsim_umma_pair1_kernel(const __grid_constant__ CUtensorMap tmap_rows, const __
         int row0 = 0;  // dummy tile once this stream is exhausted
         if (k & 1) {
           if (w1.valid(n_units)) {
-            row0 = (w1.c0 + 4 * w1.t) * kGroup;
+            row0 = w1.chunk() * kGroup;
             w1.next(unit_start, unit_end, n_units);
           }
         } else if (w0.valid(n_units)) {
-          row0 = (w0.c0 + 4 * w0.t) * kGroup;
+          row0 = w0.chunk() * kGroup;
           w0.next(unit_start, unit_end, n_units);
         }
-        mbar_wait(&empty[stage], phase ^ 1);
-        if (rank == 0) mbar_expect_tx(&full[stage], 2 * K::kTileBytes);
-        uint8_t* dst = smem_st + size_t(stage) * K::kTileBytes;
+        mbar_wait(&sm.empty[stage], phase ^ 1);
+        if (rank == 0) mbar_expect_tx(&sm.full[stage], 2 * K::kTileBytes);
+        uint8_t* dst = sm.st + size_t(stage) * K::kTileBytes;
 #pragma unroll
         for (int p = 0; p < K::kPanels; ++p)
           tma_load_2d_pair(&tmap_rows, full_l + uint32_t(stage) * 8u, dst + p * kSubtileBytes, p * K::kPanelElems, row0,
@@ -402,7 +271,7 @@ maxsim_umma_pair1_kernel(const __grid_constant__ CUtensorMap tmap_rows, const __
         }
       }
       for (int i = 0; i < num_stages; ++i) {  // tail: let the last multicast commits land before this CTA may exit
-        mbar_wait(&empty[stage], phase ^ 1);
+        mbar_wait(&sm.empty[stage], phase ^ 1);
         if (++stage == num_stages) {
           stage = 0;
           phase ^= 1;
@@ -413,27 +282,21 @@ maxsim_umma_pair1_kernel(const __grid_constant__ CUtensorMap tmap_rows, const __
     if (rank == 0) {
       constexpr uint32_t idesc = umma_idesc(KIND, 2 * kTileM, kPairN);
       constexpr uint32_t kTileDesc = K::kTileBytes >> 4;
-      mbar_wait(qfull, 0);
+      mbar_wait(sm.qfull, 0);
       tc_fence_after();
-      const uint64_t ad = umma_desc_kmajor_sw128(smem_u32(smem_q));
-      const uint64_t b_desc0 = umma_desc_kmajor_sw128(smem_u32(smem_st));
+      const uint64_t ad = umma_desc_kmajor_sw128(smem_u32(sm.q));
+      const uint64_t b_desc0 = umma_desc_kmajor_sw128(smem_u32(sm.st));
       int stage = 0;
       uint32_t phase = 0;
       for (int k = 0; k < n_iter; ++k) {
         const uint32_t buf = k & 1;
-        mbar_wait(&full[stage], phase);
-        mbar_wait(&tempty[buf], ((uint32_t(k) >> 1) & 1) ^ 1);
+        mbar_wait(&sm.full[stage], phase);
+        mbar_wait(&sm.tempty[buf], ((uint32_t(k) >> 1) & 1) ^ 1);
         tc_fence_after();
         if (elect_one()) {
-          const uint32_t d_tmem = tmem_base + buf * kPairN;
-          const uint64_t bd = b_desc0 + uint64_t(uint32_t(stage) * kTileDesc);
-#pragma unroll
-          for (int ks = 0; ks < kKSteps; ++ks) {
-            const uint32_t off = ((ks >> 2) * kSubtileBytes + (ks & 3) * 32) >> 4;
-            umma2_ss<KIND>(d_tmem, ad + off, bd + off, idesc, ks != 0);
-          }
-          umma2_commit_mc(&tfull[buf], 3);
-          umma2_commit_mc(&empty[stage], 3);
+          umma_tile<KIND, true>(tmem_base + buf * kPairN, ad, b_desc0 + uint64_t(uint32_t(stage) * kTileDesc), idesc);
+          umma2_commit_mc(&sm.tfull[buf], 3);
+          umma2_commit_mc(&sm.empty[stage], 3);
         }
         __syncwarp();
         if (++stage == num_stages) {
@@ -448,131 +311,41 @@ maxsim_umma_pair1_kernel(const __grid_constant__ CUtensorMap tmap_rows, const __
     const int half = e & 1;  // column half = CTA whose producer loaded these rows
     const int quad = warp & 3;
     const uint32_t taddr = tmem_base + (uint32_t(quad * 32) << 16) + buf * kPairN + half * kTileN;
-    const uint32_t tempty_l = mapa_rank(smem_u32(&tempty[buf]), 0);
+    const uint32_t tempty_l = mapa_rank(smem_u32(&sm.tempty[buf]), 0);
+    const auto release = [&] { mbar_arrive_cluster(tempty_l); };
     const int group = (m_tile_base + int(rank)) * 4 + quad;
     UnitWalk w;
     w.init(stream0 + 2 * half + buf, vstride, unit_start, unit_end, n_units);
-    Acc runmax = Acc{};
-    int cur_page = -1, last_u = -1;
+    PageRun<Acc> run;
+    int last_u = -1;
+    const auto emit = [&](int page, Acc rm) {
+      store_group_score(group_scores, ld, group, slot_mode ? last_u : page, clamp_bits, rm);
+    };
     for (int n = 0; n < n_half; ++n) {
-      mbar_wait(&tfull[buf], n & 1);
+      mbar_wait(&sm.tfull[buf], n & 1);
       tc_fence_after();
       if (group < n_groups_real && w.valid(n_units)) {
         if (w.u != last_u) {  // a new unit starts: units are whole pages
-          if (cur_page >= 0) {
-            const int o = slot_mode ? last_u : cur_page;
-            const Acc s2 = warp_sum(clamp_token_max(clamp_bits, o, runmax));
-            if (lane == 0) group_scores[int64_t(group) * ld + o] = s2;
-          }
-          cur_page = -1;
+          run.flush(emit);
           last_u = w.u;
         }
-        const int cb = w.c0 + 4 * w.t;
         int pg[4];
-#pragma unroll
-        for (int j = 0; j < 4; ++j) pg[j] = (cb + j < w.c1) ? __ldg(chunk_page + cb + j) : -1;
-        uint32_t va[32], vb[32];
+        tile_pages(chunk_page, w.chunk(), w.c1, pg);
         Acc cm[4];
-        tmem_ld_32x32(taddr, va);
-        tmem_ld_32x32(taddr + 32, vb);
-        tmem_ld_wait();
-        cm[0] = chunk_max<Acc>(va);
-        cm[1] = chunk_max<Acc>(vb);
-        tmem_ld_32x32(taddr + 64, va);
-        tmem_ld_32x32(taddr + 96, vb);
-        tmem_ld_wait();
-        tc_fence_before();
-        __syncwarp();
-        if (lane == 0) mbar_arrive_cluster(tempty_l);
-        cm[2] = chunk_max<Acc>(va);
-        cm[3] = chunk_max<Acc>(vb);
-#pragma unroll
-        for (int j = 0; j < 4; ++j) {
-          if (pg[j] < 0) continue;
-          if (pg[j] != cur_page) {
-            if (cur_page >= 0) {
-              const int o = slot_mode ? last_u : cur_page;
-              const Acc s2 = warp_sum(clamp_token_max(clamp_bits, o, runmax));
-              if (lane == 0) group_scores[int64_t(group) * ld + o] = s2;
-            }
-            cur_page = pg[j];
-            runmax = cm[j];
-          } else {
-            runmax = acc_max(runmax, cm[j]);
-          }
-        }
+        drain_accum(taddr, cm, release);
+        run.fold(pg, cm, emit);
         w.next(unit_start, unit_end, n_units);
       } else {
-        tc_fence_before();
-        __syncwarp();
-        if (lane == 0) mbar_arrive_cluster(tempty_l);
+        release_accum(release);
       }
     }
-    if (group < n_groups_real && cur_page >= 0) {
-      const int o = slot_mode ? last_u : cur_page;
-      const Acc s2 = warp_sum(clamp_token_max(clamp_bits, o, runmax));
-      if (lane == 0) group_scores[int64_t(group) * ld + o] = s2;
-    }
+    run.flush(emit);
   }
-
-  __syncwarp();
-  tc_fence_before();
-  cluster_sync_all();
-  if (warp == 2) {
-    tc_fence_after();
-    tmem_dealloc_512_pair(tmem_base);
-  }
+  tile_teardown<true>(warp, tmem_base);
 }
 
-template <int KIND, int NM>
-static int launch_pair(b200ms_t* h, const UnitPlan& up, const CUtensorMap& tq, int m_tile_base, int n_groups_real,
-                       void* scores, int64_t ld, cudaStream_t s) {
-  using K = Kind<KIND>;
-  const Corpus& c = h->corpus;
-  const uint32_t avail = kSmemLimit - 1024 - kBarrierBytes - NM * K::kTileBytes;
-  int stages = int(avail / K::kTileBytes);
-  if (stages > 8) stages = 8;
-  if (stages < 2) return set_error(h, B200MS_EINVAL, "maxsim_umma_pair: not enough shared memory for 2 stages");
-  const uint32_t smem = 1024 + NM * K::kTileBytes + uint32_t(stages) * K::kTileBytes + kBarrierBytes;
-  auto kern = maxsim_umma_pair_kernel<KIND, NM>;
-  if (int e = ensure_smem(h, reinterpret_cast<const void*>(kern), int(smem), "cudaFuncSetAttribute(maxsim_umma_pair)"))
-    return e;
-  if (up.n_units < 1) return B200MS_OK;
-  int grid = (h->max_ctas > 0 ? h->max_ctas : h->num_sms) & ~1;  // whole pairs
-  if (h->pair_clusters < 0) {  // once per handle: can this device co-schedule CTA pairs of this size at all?
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3(2);
-    cfg.blockDim = dim3(kThreadsPair);
-    cfg.dynamicSmemBytes = smem;
-    int n = 0;
-    const cudaError_t qe = cudaOccupancyMaxActiveClusters(&n, kern, &cfg);
-    if (qe != cudaSuccess) (void)cudaGetLastError();
-    h->pair_clusters = qe == cudaSuccess ? n : 0;
-  }
-  if (h->pair_clusters < 1) return B200MS_EUNSUPPORTED_PAIR;  // caller falls back to the one-CTA kernels (still CUDA)
-  const int want = (up.n_units + 1) & ~1;
-  if (grid > want) grid = want;
-  if (grid < 2) grid = 2;
-  kern<<<grid, kThreadsPair, smem, s>>>(c.tmap, tq, static_cast<const int32_t*>(h->chunk_page.p), up.start, up.end,
-                                       up.slot_mode, up.n_units, m_tile_base, n_groups_real, up.clamp_bits,
-                                       static_cast<typename K::Acc*>(scores), ld, stages);
-  h->launches++;
-  return check_cuda(h, cudaGetLastError(), "launch maxsim_umma_pair");
-}
-
-template <int KIND>
-static int launch_pair1(b200ms_t* h, const UnitPlan& up, const CUtensorMap& tq, int m_tile_base, int n_groups_real,
-                        void* scores, int64_t ld, cudaStream_t s) {
-  using K = Kind<KIND>;
-  const Corpus& c = h->corpus;
-  const uint32_t avail = kSmemLimit - 1024 - kBarrierBytes - K::kTileBytes;
-  int stages = int(avail / K::kTileBytes);
-  if (stages > 8) stages = 8;
-  const uint32_t smem = 1024 + K::kTileBytes + uint32_t(stages) * K::kTileBytes + kBarrierBytes;
-  auto kern = maxsim_umma_pair1_kernel<KIND>;
-  if (int e = ensure_smem(h, reinterpret_cast<const void*>(kern), int(smem), "cudaFuncSetAttribute(maxsim_umma_pair1)"))
-    return e;
-  if (up.n_units < 1) return B200MS_OK;
+// Once per handle: can this device co-schedule CTA pairs of this size at all?
+static bool pairs_schedulable(b200ms_t* h, const void* kern, uint32_t smem) {
   if (h->pair_clusters < 0) {
     cudaLaunchConfig_t cfg = {};
     cfg.gridDim = dim3(2);
@@ -583,16 +356,38 @@ static int launch_pair1(b200ms_t* h, const UnitPlan& up, const CUtensorMap& tq, 
     if (qe != cudaSuccess) (void)cudaGetLastError();
     h->pair_clusters = qe == cudaSuccess ? n : 0;
   }
-  if (h->pair_clusters < 1) return B200MS_EUNSUPPORTED_PAIR;
-  int grid = (h->max_ctas > 0 ? h->max_ctas : h->num_sms) & ~1;
-  const int want = (((up.n_units + 1) / 2) + 1) & ~1;  // two unit streams per CTA
-  if (grid > want) grid = want;
-  if (grid < 2) grid = 2;
-  kern<<<grid, kThreadsPair, smem, s>>>(c.tmap, tq, static_cast<const int32_t*>(h->chunk_page.p), up.start, up.end,
-                                       up.slot_mode, up.n_units, m_tile_base, n_groups_real, up.clamp_bits,
-                                       static_cast<typename K::Acc*>(scores), ld, stages);
-  h->launches++;
-  return check_cuda(h, cudaGetLastError(), "launch maxsim_umma_pair1");
+  return h->pair_clusters >= 1;
+}
+
+// NM = query tiles per CTA: 1 on the two-tile kernel, 2 / 4 / 8 on maxsim_umma_pair_kernel.  B200MS_EUNSUPPORTED_PAIR:
+// the device cannot co-schedule the pair, and the caller falls back to the one-CTA kernels (still CUDA).
+template <int KIND, int NM>
+static int launch_pair(b200ms_t* h, const UnitPlan& up, const CUtensorMap& tq, int m_tile_base, int n_groups_real,
+                       void* scores, int64_t ld, cudaStream_t s) {
+  using K = Kind<KIND>;
+  const uint32_t avail = kSmemLimit - 1024 - kBarrierBytes - NM * K::kTileBytes;
+  int stages = int(avail / K::kTileBytes);
+  if (stages > 8) stages = 8;
+  if (stages < 2) return set_error(h, B200MS_EINVAL, "maxsim_umma_pair: not enough shared memory for 2 stages");
+  const uint32_t smem = 1024 + NM * K::kTileBytes + uint32_t(stages) * K::kTileBytes + kBarrierBytes;
+  const auto launch = [&](auto kern, const char* name, int want) {
+    if (int e = ensure_smem(h, reinterpret_cast<const void*>(kern), int(smem), name)) return e;
+    if (up.n_units < 1) return int(B200MS_OK);
+    if (!pairs_schedulable(h, reinterpret_cast<const void*>(kern), smem)) return B200MS_EUNSUPPORTED_PAIR;
+    int grid = (h->max_ctas > 0 ? h->max_ctas : h->num_sms) & ~1;  // whole pairs
+    if (grid > want) grid = want;
+    if (grid < 2) grid = 2;
+    kern<<<grid, kThreadsPair, smem, s>>>(h->corpus.tmap, tq, static_cast<const int32_t*>(h->chunk_page.p), up.start, up.end,
+                                         up.slot_mode, up.n_units, m_tile_base, n_groups_real, up.clamp_bits,
+                                         static_cast<typename K::Acc*>(scores), ld, stages);
+    h->launches++;
+    return check_cuda(h, cudaGetLastError(), name);
+  };
+  if constexpr (NM == 1) {
+    return launch(maxsim_umma_pair1_kernel<KIND>, "maxsim_umma_pair1", (((up.n_units + 1) / 2) + 1) & ~1);  // 2 streams per CTA
+  } else {
+    return launch(maxsim_umma_pair_kernel<KIND, NM>, "maxsim_umma_pair", (up.n_units + 1) & ~1);
+  }
 }
 
 // nm = query tiles per CTA (1, 2, 4; 8 for the one-byte dtypes): one launch scores 2*nm query tiles [m_tile_base, m_tile_base + 2*nm).
@@ -600,7 +395,7 @@ template <int KIND>
 static int launch_pair_kind(b200ms_t* h, const UnitPlan& up, const CUtensorMap& tq, int nm, int m_tile_base,
                             int n_groups_real, void* scores, int64_t ld, cudaStream_t s) {
   switch (nm) {
-    case 1: return launch_pair1<KIND>(h, up, tq, m_tile_base, n_groups_real, scores, ld, s);
+    case 1: return launch_pair<KIND, 1>(h, up, tq, m_tile_base, n_groups_real, scores, ld, s);
     case 2: return launch_pair<KIND, 2>(h, up, tq, m_tile_base, n_groups_real, scores, ld, s);
     case 4: return launch_pair<KIND, 4>(h, up, tq, m_tile_base, n_groups_real, scores, ld, s);
     case 8:

@@ -1,5 +1,5 @@
-// umma_tile.cuh -- tile geometry and accumulator helpers shared by the tcgen05 MaxSim kernels
-// (maxsim_umma.cu: one CTA per SM; maxsim_umma_pair.cu: CTA pairs, cta_group::2).
+// umma_tile.cuh -- tile geometry, pipeline pieces and accumulator helpers shared by the query-as-M tcgen05 MaxSim kernels
+// (maxsim_umma.cu: one CTA per SM; maxsim_umma_pair.cu: CTA pairs, cta_group::2; maxsim_b1_umma.cu: 1-bit rows).
 #pragma once
 #include <type_traits>
 
@@ -80,6 +80,209 @@ template <typename Acc>
 __device__ __forceinline__ Acc clamp_token_max(const uint32_t* __restrict__ clamp_bits, int idx, Acc rm) {
   if (clamp_bits != nullptr && ((__ldg(clamp_bits + (idx >> 5)) >> (idx & 31)) & 1u)) return acc_max(rm, Acc(0));
   return rm;
+}
+
+// ---------------------------------------------------------------------------------------------- CTA layout and lifetime
+// Dynamic shared memory: [1024-aligned] resident query tiles | num_stages patch tiles | kBarrierBytes of barriers.
+struct TileSmem {
+  uint8_t* q;
+  uint8_t* st;
+  uint64_t* full;    // [num_stages] producer -> MMA
+  uint64_t* empty;   // [num_stages] MMA -> producer
+  uint64_t* tfull;   // [accumulators] MMA -> epilogue
+  uint64_t* tempty;  // [accumulators] epilogue -> MMA
+  uint64_t* qfull;   // query tiles landed
+  uint32_t* tmem_slot;
+};
+
+__device__ __forceinline__ TileSmem carve_tile_smem(uint8_t* raw, uint32_t q_bytes, uint32_t tile_bytes, int num_stages) {
+  TileSmem sm;
+  sm.q = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(raw) + 1023) & ~uintptr_t(1023));
+  sm.st = sm.q + q_bytes;
+  uint64_t* bars = reinterpret_cast<uint64_t*>(sm.st + size_t(num_stages) * tile_bytes);
+  sm.full = bars;
+  sm.empty = bars + 16;
+  sm.tfull = bars + 32;
+  sm.tempty = bars + 40;
+  sm.qfull = bars + 48;
+  sm.tmem_slot = reinterpret_cast<uint32_t*>(bars + 56);
+  return sm;
+}
+
+// Thread 0 prefetches the tensor maps (tmap_b may be null) and initialises the barriers, warp 2 allocates all 512 TMEM
+// columns, and the CTA (PAIR: the cluster) synchronises so both are visible before any arrive or TMA signal.
+template <bool PAIR>
+__device__ __forceinline__ uint32_t tile_prologue(const TileSmem& sm, int warp, const CUtensorMap* tmap_a,
+                                                  const CUtensorMap* tmap_b, int num_stages, uint32_t full_count, int n_accum,
+                                                  uint32_t tempty_count) {
+  if (threadIdx.x == 0) {
+    prefetch_tmap(tmap_a);
+    if (tmap_b != nullptr) prefetch_tmap(tmap_b);
+    for (int i = 0; i < num_stages; ++i) {
+      mbar_init(&sm.full[i], full_count);
+      mbar_init(&sm.empty[i], 1);
+    }
+    for (int i = 0; i < n_accum; ++i) {
+      mbar_init(&sm.tfull[i], 1);
+      mbar_init(&sm.tempty[i], tempty_count);
+    }
+    mbar_init(sm.qfull, 1);
+    fence_mbar_init();
+  }
+  if (warp == 2) {
+    if constexpr (PAIR) tmem_alloc_512_pair(sm.tmem_slot);
+    else tmem_alloc_512(sm.tmem_slot);
+  }
+  tc_fence_before();
+  if constexpr (PAIR) cluster_sync_all();
+  else __syncthreads();
+  tc_fence_after();
+  return *sm.tmem_slot;
+}
+
+// Nobody exits (or frees TMEM) while another warp -- PAIR: the partner CTA -- can still touch shared memory or TMEM.
+template <bool PAIR>
+__device__ __forceinline__ void tile_teardown(int warp, uint32_t tmem_base) {
+  if constexpr (PAIR) __syncwarp();
+  tc_fence_before();
+  if constexpr (PAIR) cluster_sync_all();
+  else __syncthreads();
+  if (warp == 2) {
+    tc_fence_after();
+    if constexpr (PAIR) tmem_dealloc_512_pair(tmem_base);
+    else tmem_dealloc_512(tmem_base);
+  }
+}
+
+// ---------------------------------------------------------------------------------------------- MMA issue
+// One 128-deep contraction into d_tmem: K::kKSteps tcgen05.mma of 32 B of K each, four per 128 B panel; ad / bd describe
+// the first panel of the A / B tile.  PAIR issues the cta_group::2 form.
+template <int KIND, bool PAIR = false>
+__device__ __forceinline__ void umma_tile(uint32_t d_tmem, uint64_t ad, uint64_t bd, uint32_t idesc) {
+#pragma unroll
+  for (int ks = 0; ks < Kind<KIND>::kKSteps; ++ks) {
+    const uint32_t off = ((ks >> 2) * kSubtileBytes + (ks & 3) * 32) >> 4;
+    if constexpr (PAIR) umma2_ss<KIND>(d_tmem, ad + off, bd + off, idesc, ks != 0);
+    else umma_ss<KIND>(d_tmem, ad + off, bd + off, idesc, ks != 0);
+  }
+}
+
+// ---------------------------------------------------------------------------------------------- epilogue
+// Hand an accumulator back to the MMA warp; release() is the arrive on tempty (local, or on the leader CTA's barrier).
+template <typename Release>
+__device__ __forceinline__ void release_accum(Release&& release) {
+  tc_fence_before();
+  __syncwarp();
+  if ((threadIdx.x & 31) == 0) release();
+}
+
+// Drain the 128 columns of one accumulator in this warp's lane quadrant: cm[j] = the thread's maximum over chunk j.  Two
+// loads stay in flight, and the accumulator is released as soon as the last one has landed, before the last two maxima.
+template <typename Acc, typename Release>
+__device__ __forceinline__ void drain_accum(uint32_t taddr, Acc (&cm)[4], Release&& release) {
+  uint32_t va[32], vb[32];
+  tmem_ld_32x32(taddr, va);
+  tmem_ld_32x32(taddr + 32, vb);
+  tmem_ld_wait();
+  cm[0] = chunk_max<Acc>(va);
+  cm[1] = chunk_max<Acc>(vb);
+  tmem_ld_32x32(taddr + 64, va);
+  tmem_ld_32x32(taddr + 96, vb);
+  tmem_ld_wait();
+  release_accum(release);
+  cm[2] = chunk_max<Acc>(va);
+  cm[3] = chunk_max<Acc>(vb);
+}
+
+// pg[j] = page of chunk cb + j of a tile, or -1 past the unit's last chunk c1
+__device__ __forceinline__ void tile_pages(const int32_t* __restrict__ chunk_page, int cb, int c1, int (&pg)[4]) {
+#pragma unroll
+  for (int j = 0; j < 4; ++j) pg[j] = (cb + j < c1) ? __ldg(chunk_page + cb + j) : -1;
+}
+
+// One closed (group, page) run of the bf16 / int8 / fp8 kernels: zero_pad_compat clamp, 32-token sum, lane 0 stores column o.
+template <typename Acc>
+__device__ __forceinline__ void store_group_score(Acc* __restrict__ group_scores, int64_t ld, int group, int o,
+                                                  const uint32_t* __restrict__ clamp_bits, Acc rm) {
+  const Acc s = warp_sum(clamp_token_max(clamp_bits, o, rm));
+  if ((threadIdx.x & 31) == 0) group_scores[int64_t(group) * ld + o] = s;
+}
+
+// The running per-token max of one query group over its open page.  Units hold whole pages, so a page closes either at a
+// page change inside fold() or at the unit's end (flush()).  emit(page, rm) writes one closed page: the kernel's output
+// index, clamp, 32-token warp sum and lane-0 store.
+template <typename Acc>
+struct PageRun {
+  Acc rm;
+  int cp = -1;  // open page, -1: none
+
+  template <typename Emit>
+  __device__ __forceinline__ void fold(const int (&pg)[4], const Acc (&cm)[4], Emit&& emit) {
+#pragma unroll
+    for (int j = 0; j < 4; ++j) {
+      if (pg[j] < 0) continue;  // chunk belongs to the next unit
+      if (pg[j] != cp) {
+        if (cp >= 0) emit(cp, rm);
+        cp = pg[j];
+        rm = cm[j];
+      } else {
+        rm = acc_max(rm, cm[j]);
+      }
+    }
+  }
+  template <typename Emit>
+  __device__ __forceinline__ void flush(Emit&& emit) {
+    if (cp >= 0) emit(cp, rm);
+    cp = -1;
+  }
+};
+
+// One stream of work units u, u + stride, ... walked one 128-row tile (4 chunks) at a time, skipping empty units.
+struct UnitWalk {
+  int u, stride, c0, c1, t, n_tiles;
+  __device__ __forceinline__ void load(const int32_t* us, const int32_t* ue, int n_units) {
+    n_tiles = 0;
+    while (u < n_units) {
+      c0 = __ldg(us + u);
+      c1 = __ldg(ue + u);
+      n_tiles = (c1 - c0 + 3) >> 2;
+      if (n_tiles > 0) break;
+      u += stride;
+    }
+    t = 0;
+  }
+  __device__ __forceinline__ void init(int v, int stride_, const int32_t* us, const int32_t* ue, int n_units) {
+    u = v;
+    stride = stride_;
+    load(us, ue, n_units);
+  }
+  __device__ __forceinline__ bool valid(int n_units) const { return u < n_units; }
+  __device__ __forceinline__ int chunk() const { return c0 + 4 * t; }  // first chunk of the current tile
+  __device__ __forceinline__ void next(const int32_t* us, const int32_t* ue, int n_units) {
+    if (++t == n_tiles) {
+      u += stride;
+      load(us, ue, n_units);
+    }
+  }
+};
+
+// ---------------------------------------------------------------------------------------------- host side
+// Persistent one-CTA launch: a ring of as many tile_bytes stages as fit beside resident_bytes in the 227 KB opt-in (at most
+// max_stages, at least 2), grid = one CTA per SM (or max_ctas), at most one per unit.  num_stages is the kernel's last argument.
+template <typename... Params, typename... Args>
+static int launch_persistent(b200ms_t* h, void (*kern)(Params...), const char* name, int threads, uint32_t resident_bytes,
+                             uint32_t tile_bytes, int max_stages, int n_units, cudaStream_t s, Args... args) {
+  int stages = int((kSmemLimit - 1024 /*align*/ - kBarrierBytes - resident_bytes) / tile_bytes);
+  if (stages > max_stages) stages = max_stages;
+  if (stages < 2) return set_error(h, B200MS_EINVAL, std::string(name) + ": not enough shared memory for 2 stages");
+  const uint32_t smem = 1024 + resident_bytes + uint32_t(stages) * tile_bytes + kBarrierBytes;
+  if (int e = ensure_smem(h, reinterpret_cast<const void*>(kern), int(smem), name)) return e;
+  int grid = h->max_ctas > 0 ? h->max_ctas : h->num_sms;
+  if (grid > n_units) grid = n_units;
+  if (grid < 1) return B200MS_OK;
+  kern<<<grid, threads, smem, s>>>(args..., stages);
+  h->launches++;
+  return check_cuda(h, cudaGetLastError(), name);
 }
 
 }  // namespace bms

@@ -284,8 +284,8 @@ def test_int8_bit_exact(n_q):
     lens = [1, 33, 0, 64, 200, 1024, 17, 96] + list(rng.integers(1, 260, size=30))
     pages = make_pages(rng, lens)
     queries = [unit_rows(rng, 32 if i % 3 else 19) for i in range(n_q)]
-    # every dot product of these tokens is negative (all-negative query x all-positive pages below): the per-chunk maximum
-    # is negative, which the epilogue's float-datapath max cannot order -> its exact integer fallback must kick in
+    # every dot product of these tokens is negative (all-negative query x all-positive pages below), so every per-chunk maximum
+    # is a negative int32: the epilogue's integer max must order those exactly (a float max over the bit patterns would not)
     queries[0] = -np.abs(queries[0])
     for j in (3, 4, 9):
         pages[j] = np.abs(pages[j])
@@ -331,7 +331,9 @@ def test_binary_known_answers_from_reference_tests(golden_dir):
         assert ti[0][0] == j and ts[0][0] == 3.0 and np.all(np.diff(ts[0]) <= 0)
 
 
-@pytest.mark.parametrize("path", [0, 1, 2])  # 0 = POPC kernel, 1 = tcgen05 kernel (incl. the replicated-query form), 2 = auto
+# 0 = POPC kernel, 1 = tcgen05 kernels, 2 = auto.  With the default rowm = 1, paths 1 and 2 send a scan of ONE 32-token group
+# to the rows-as-M kernel (maxsim_rowm.cu); "query_as_m" is path 1 with rowm = 0, so that scan runs on maxsim_b1_umma_kernel<1>.
+@pytest.mark.parametrize("path", [0, 1, 2, "query_as_m"])
 @pytest.mark.parametrize("n_q", [1, 3, 8, 13])
 def test_binary_bit_exact(n_q, path):
     rng = np.random.default_rng(50 + n_q)
@@ -339,6 +341,9 @@ def test_binary_bit_exact(n_q, path):
     pages = make_pages(rng, lens)
     queries = [unit_rows(rng, t) for t in ([32, 7, 45, 1, 20, 64, 33, 32, 2, 9, 100, 31, 32][:n_q])]
     idx = MaxSimIndex(dtype="binary")
+    if path == "query_as_m":
+        idx.set_option("rowm", 0)
+        path = 1
     idx.set_option("b1_tensor", path)
     idx.add_pages(pages)
     got = idx.score_matrix(queries)
