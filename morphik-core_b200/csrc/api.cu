@@ -144,6 +144,26 @@ int make_tmap_rows(b200ms_t* h, CUtensorMap* out, const void* base, int dtype, i
   return B200MS_OK;
 }
 
+int query_tmap(b200ms_t* h, const void* base, int dtype, int64_t n_rows, int box_rows, const CUtensorMap** out) {
+  QueryTmaps& c = h->query_tmaps;
+  for (QueryTmaps::Entry& en : c.slot) {
+    if (en.base == base && en.dtype == dtype && en.rows == n_rows && en.box_rows == box_rows) {
+      *out = &en.map;
+      return B200MS_OK;
+    }
+  }
+  QueryTmaps::Entry& en = c.slot[c.next];
+  en.dtype = -1;
+  if (int e = make_tmap_rows(h, &en.map, base, dtype, n_rows, box_rows)) return e;
+  en.base = base;
+  en.dtype = dtype;
+  en.rows = n_rows;
+  en.box_rows = box_rows;
+  c.next = (c.next + 1) % QueryTmaps::kSlots;
+  *out = &en.map;
+  return B200MS_OK;
+}
+
 static bool corpus_dtype_ok(int d) { return d == B200MS_BF16 || d == B200MS_I8 || d == B200MS_B1 || d == B200MS_F8; }
 static bool src_dtype_ok(int d) { return d == B200MS_F32 || d == B200MS_BF16; }
 
@@ -241,7 +261,6 @@ B200MS_API int b200ms_create(int device, b200ms_t** out) {
   if (const char* e = getenv("B200MS_B1_TENSOR")) h->b1_tensor = atoi(e);
   if (const char* e = getenv("B200MS_PAIR_CTA")) h->pair_cta = atoi(e);
   if (const char* e = getenv("B200MS_ROWM")) h->rowm = atoi(e) != 0;
-  if (const char* e = getenv("B200MS_ROWM_FAST")) h->rowm_fast_path = atoi(e);
   if (const char* e = getenv("B200MS_ZERO_COPY")) h->zero_copy = atoi(e);
   if (const char* e = getenv("B200MS_UNIT_ROWS")) { if (atoll(e) > 0) h->unit_rows = atoll(e); }
   if (int e = check_cuda(h, cudaStreamCreateWithFlags(&h->stream, cudaStreamNonBlocking), "cudaStreamCreate")) {
@@ -619,7 +638,7 @@ static int score_impl(b200ms_t* h, const void* q_packed, int n_groups, const int
       sub.n_units = int(int64_t(q_hi - q_lo) * cs.stride);
       if (sub.clamp_bits) sub.clamp_bits += s0 / 32;
       void* sc = static_cast<uint8_t*>(group_scores) + size_t(s0) * 4;
-      if (int e = launch_score_umma(h, &sub, q_packed, n_groups, sc, ld, s, m, m + 1)) return e;
+      if (int e = launch_score_umma(h, &sub, q_packed, n_groups, sc, ld, s, m)) return e;
     }
   } else if (!cs.ids && h->rowm && n_groups <= kRowmMaxGroups) {
     // the lone query: patch rows as the M operand, four epilogue warps in parallel (maxsim_rowm.cu)

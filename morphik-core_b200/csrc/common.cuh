@@ -65,6 +65,21 @@ struct Corpus {
   int64_t clamp_batch = 0;  // zero_pad_compat batch size the full-scan clamp bitmask (b200ms::clamp_pages) was built for
 };
 
+// Tensor maps of the query rows of the scoring launches (query_tmap), keyed on everything such a map encodes.  A map
+// depends on nothing else, so an entry never goes stale; a miss re-encodes into the oldest slot.
+struct QueryTmaps {
+  struct Entry {
+    const void* base = nullptr;
+    int dtype = -1;  // -1: empty slot
+    int64_t rows = 0;
+    int box_rows = 0;
+    CUtensorMap map;
+  };
+  static constexpr int kSlots = 4;  // a scoring call needs one map; a miss costs one host-side encode
+  Entry slot[kSlots];
+  int next = 0;  // slot the next miss fills
+};
+
 }  // namespace bms
 
 struct b200ms {
@@ -110,16 +125,7 @@ struct b200ms {
   int pair_cta = 2;   // CTA-pair kernels (cta_group::2, maxsim_umma_pair.cu): 0 off, 1 for passes of >= 3 query tiles, 2 (default) also for 2 tiles
   int pair_clusters = -1;  // co-resident CTA pairs the device reports for the pair kernel (-1: not queried yet)
   int zero_pad_batch = 0;  // > 0: reproduce score_multi_vector's zero-padding quirk with this batch size (128 upstream)
-  CUtensorMap tmap_q;  // query tiles; re-encoded only when (pointer, dtype, rows) change
-  const void* tmap_q_base = nullptr;
-  int tmap_q_dtype = -1;
-  int64_t tmap_q_rows = -1;
-  CUtensorMap tmap_qn;  // the same query rows as a 32*NG-row box (maxsim_rowm.cu: the query is the N operand)
-  const void* tmap_qn_base = nullptr;
-  int tmap_qn_dtype = -1;
-  int64_t tmap_qn_rows = -1;
-  int tmap_qn_box = 0;
-  int rowm_fast_path = 1;   // A/B knob (env B200MS_ROWM_FAST): epilogue fast path for 8-tile blocks inside one page (A/B: faster for every dtype)
+  bms::QueryTmaps query_tmaps;
   int rowm = 1;  // option "rowm": full scans of <= kRowmMaxGroups query groups run on maxsim_rowm_kernel (0: query-as-M kernels)
   // CUDA graphs of the small zero-copy host search (pack -> score -> top-k): key -> executable graph
   struct HostGraph {
@@ -150,6 +156,8 @@ int reserve_pinned(b200ms_t* h, PinnedBuf& b, size_t bytes);
 int ensure_smem(b200ms_t* h, const void* kernel, int smem, const char* what);
 int make_tmap_rows(b200ms_t* h, CUtensorMap* out, const void* base, int dtype, int64_t n_rows, int box_rows,
                    int64_t row_bytes = 0);
+// make_tmap_rows of query rows (default row bytes) through the handle's QueryTmaps; a later call may re-encode *out
+int query_tmap(b200ms_t* h, const void* base, int dtype, int64_t n_rows, int box_rows, const CUtensorMap** out);
 void comm_teardown(b200ms_t* h);
 // pack -> score -> top-k on stream s (api.cu); meta_in_place / meta_host_block: see the definition
 int search_core(b200ms_t* h, const void* q_src, int src_dtype, const int32_t* q_lens, int n_q, int k,
@@ -159,7 +167,7 @@ int search_core(b200ms_t* h, const void* q_src, int src_dtype, const int32_t* q_
 
 // kernel launchers (each returns a b200ms error code and bumps h->launches)
 int launch_score_umma(b200ms_t* h, const UnitPlan* plan, const void* q_packed, int n_groups_real, void* group_scores,
-                      int64_t ld, cudaStream_t s, int m_tile_lo = 0, int m_tile_hi = -1);
+                      int64_t ld, cudaStream_t s, int m_tile = -1);
 constexpr int B200MS_EUNSUPPORTED_PAIR = -100;  // internal: pair kernel cannot be scheduled on this device
 int launch_score_umma_pair(b200ms_t* h, const UnitPlan& up, const CUtensorMap& tq, int nm, int m_tile_base,
                            int n_groups_real, void* scores, int64_t ld, cudaStream_t s);

@@ -24,6 +24,7 @@
 
 #include "common.cuh"
 #include "ptx.cuh"
+#include "umma_tile.cuh"
 
 namespace bms {
 
@@ -260,36 +261,12 @@ fde_scan_umma_kernel(const __grid_constant__ CUtensorMap tmap_f, const __grid_co
   const uint32_t b_bytes = uint32_t(nqp) * 128u;
   const uint32_t stage_bytes = kScanATile + b_bytes;    // multiples of 1024 (nqp % 32 == 0)
   extern __shared__ uint8_t smem_raw[];
-  uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
-  uint64_t* bars = reinterpret_cast<uint64_t*>(smem + size_t(num_stages) * stage_bytes);
-  uint64_t* full = bars;         // [num_stages] TMA -> MMA
-  uint64_t* empty = bars + 16;   // [num_stages] MMA -> TMA
-  uint64_t* tfull = bars + 32;   // [2] MMA -> epilogue
-  uint64_t* tempty = bars + 34;  // [2] epilogue -> MMA
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + 40);
-
+  const TileSmem sm = carve_tile_smem(smem_raw, 0, stage_bytes, num_stages);  // stage = A tile | B (queries)
   const int warp = threadIdx.x >> 5;
   const int lane = threadIdx.x & 31;
   const int64_t n_tiles = (n_pages + 127) / 128;
-
-  if (warp == 0 && lane == 0) {
-    prefetch_tmap(&tmap_f);
-    prefetch_tmap(&tmap_q);
-    for (int i = 0; i < num_stages; ++i) {
-      mbar_init(&full[i], 1);
-      mbar_init(&empty[i], 1);
-    }
-    for (int i = 0; i < 2; ++i) {
-      mbar_init(&tfull[i], 1);
-      mbar_init(&tempty[i], 4);
-    }
-    fence_mbar_init();
-  }
-  if (warp == 2) tmem_alloc_512(tmem_slot);
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  const uint32_t tmem_base = *tmem_slot;
+  // two accumulators; tempty: one arrive per epilogue warp
+  const uint32_t tmem_base = tile_prologue<false>(sm, warp, &tmap_f, &tmap_q, num_stages, 1, 2, 4);
 
   if (warp == 0) {
     if (lane == 0) {
@@ -299,11 +276,11 @@ fde_scan_umma_kernel(const __grid_constant__ CUtensorMap tmap_f, const __grid_co
       uint32_t phase = 0;
       for (int64_t tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
         for (int kb = 0; kb < n_kblocks; ++kb) {
-          mbar_wait(&empty[stage], phase ^ 1);
-          mbar_expect_tx(&full[stage], stage_bytes);
-          uint8_t* a = smem + size_t(stage) * stage_bytes;
-          tma_load_2d(&tmap_f, &full[stage], a, kb * 64, int32_t(tile * 128), pol_f);
-          tma_load_2d(&tmap_q, &full[stage], a + kScanATile, kb * 64, 0, pol_q);
+          mbar_wait(&sm.empty[stage], phase ^ 1);
+          mbar_expect_tx(&sm.full[stage], stage_bytes);
+          uint8_t* a = sm.st + size_t(stage) * stage_bytes;
+          tma_load_2d(&tmap_f, &sm.full[stage], a, kb * 64, int32_t(tile * 128), pol_f);
+          tma_load_2d(&tmap_q, &sm.full[stage], a + kScanATile, kb * 64, 0, pol_q);
           if (++stage == num_stages) {
             stage = 0;
             phase ^= 1;
@@ -318,20 +295,20 @@ fde_scan_umma_kernel(const __grid_constant__ CUtensorMap tmap_f, const __grid_co
     uint32_t t = 0;
     for (int64_t tile = blockIdx.x; tile < n_tiles; tile += gridDim.x, ++t) {
       const uint32_t buf = t & 1;
-      mbar_wait(&tempty[buf], ((t >> 1) & 1) ^ 1);
+      mbar_wait(&sm.tempty[buf], ((t >> 1) & 1) ^ 1);
       tc_fence_after();
       const uint32_t d_tmem = tmem_base + buf * 256;
       for (int kb = 0; kb < n_kblocks; ++kb) {
-        mbar_wait(&full[stage], phase);
+        mbar_wait(&sm.full[stage], phase);
         tc_fence_after();
         if (elect_one()) {
-          const uint32_t a_addr = smem_u32(smem + size_t(stage) * stage_bytes);
+          const uint32_t a_addr = smem_u32(sm.st + size_t(stage) * stage_bytes);
           const uint64_t ad = umma_desc_kmajor_sw128(a_addr);
           const uint64_t bd = umma_desc_kmajor_sw128(a_addr + kScanATile);
 #pragma unroll
           for (int ks = 0; ks < 4; ++ks) umma_ss<0>(d_tmem, ad + ks * 2, bd + ks * 2, idesc, (kb | ks) != 0);
-          umma_commit(&empty[stage]);
-          if (kb == n_kblocks - 1) umma_commit(&tfull[buf]);
+          umma_commit(&sm.empty[stage]);
+          if (kb == n_kblocks - 1) umma_commit(&sm.tfull[buf]);
         }
         __syncwarp();
         if (++stage == num_stages) {
@@ -348,7 +325,7 @@ fde_scan_umma_kernel(const __grid_constant__ CUtensorMap tmap_f, const __grid_co
       const uint32_t buf = t & 1;
       const int64_t p = tile * 128 + quad * 32 + lane;
       const float inv = p < n_pages ? __ldg(inv_norm + p) : 0.f;
-      mbar_wait(&tfull[buf], (t >> 1) & 1);
+      mbar_wait(&sm.tfull[buf], (t >> 1) & 1);
       tc_fence_after();
       const uint32_t taddr = lane_base + buf * 256;
       if (half_cols == 16) {  // <= 16 queries: hi and lo halves sit in one 32-column load
@@ -357,7 +334,7 @@ fde_scan_umma_kernel(const __grid_constant__ CUtensorMap tmap_f, const __grid_co
         tmem_ld_wait();
         tc_fence_before();
         __syncwarp();
-        if (lane == 0) mbar_arrive(&tempty[buf]);
+        if (lane == 0) mbar_arrive(&sm.tempty[buf]);
         if (p < n_pages) {
 #pragma unroll
           for (int q = 0; q < 16; ++q)
@@ -372,7 +349,7 @@ fde_scan_umma_kernel(const __grid_constant__ CUtensorMap tmap_f, const __grid_co
           if (c + 32 >= half_cols) {  // last chunk read: the accumulator may be overwritten
             tc_fence_before();
             __syncwarp();
-            if (lane == 0) mbar_arrive(&tempty[buf]);
+            if (lane == 0) mbar_arrive(&sm.tempty[buf]);
           }
           if (p < n_pages) {
 #pragma unroll
@@ -383,13 +360,7 @@ fde_scan_umma_kernel(const __grid_constant__ CUtensorMap tmap_f, const __grid_co
       }
     }
   }
-
-  tc_fence_before();
-  __syncthreads();
-  if (warp == 2) {
-    tc_fence_after();
-    tmem_dealloc_512(tmem_base);
-  }
+  tile_teardown<false>(warp, tmem_base);
 }
 
 // q_fde fp32 [n_q, fde_dim] (queries q_base ..) -> bf16 [2*half_cols, fde_dim]: rows [0,n) hi, rows [H, H+n) lo, rest zero
@@ -473,17 +444,10 @@ int launch_fde_scan(b200ms_t* h, const void* F, const float* inv_norm, int64_t n
     if (int e = check_cuda(h, cudaGetLastError(), "launch fde_q_split")) return e;
     CUtensorMap tq;
     if (int e = make_tmap_rows(h, &tq, qb16, B200MS_BF16, nqp, nqp, int64_t(fd) * 2)) return e;
-    const uint32_t stage_bytes = kScanATile + uint32_t(nqp) * 128u;
-    int stages = int((232448u - 1024u - 1024u) / stage_bytes);
-    if (stages > 12) stages = 12;
-    const uint32_t smem = 1024 + uint32_t(stages) * stage_bytes + 1024;
-    if (int e = ensure_smem(h, reinterpret_cast<const void*>(fde_scan_umma_kernel), int(smem), "cudaFuncSetAttribute(fde_scan_umma)"))
+    const int n_tiles = int((n_pages + 127) / 128);
+    if (int e = launch_persistent(h, fde_scan_umma_kernel, "fde_scan_umma", kScanThreads, 0, kScanATile + uint32_t(nqp) * 128u,
+                                  12, n_tiles, s, tf, tq, inv_norm, n_pages, fd / 64, n_here, qb, half, scores, ld))
       return e;
-    const int64_t n_tiles = (n_pages + 127) / 128;
-    const int grid = int(n_tiles < h->num_sms ? n_tiles : h->num_sms);
-    fde_scan_umma_kernel<<<grid, kScanThreads, smem, s>>>(tf, tq, inv_norm, n_pages, fd / 64, n_here, qb, half, scores, ld, stages);
-    h->launches++;
-    if (int e = check_cuda(h, cudaGetLastError(), "launch fde_scan_umma")) return e;
   }
   return B200MS_OK;
 }

@@ -255,17 +255,17 @@ int launch_score_b1_umma(b200ms_t* h, const void* q_bits, const int32_t* group_n
   h->launches++;
   if (int e = check_cuda(h, cudaGetLastError(), "launch b1_query_expand")) return e;
   const int n_mtiles = n_groups_padded / 4;
-  h->tmap_q_base = nullptr;  // tmap_q now describes q_i8: the next bf16 / int8 / fp8 scan must re-encode it
-  if (int e = make_tmap_rows(h, &h->tmap_q, q_i8, B200MS_I8, n_rows, kTileM)) return e;
+  const CUtensorMap* tq;
+  if (int e = query_tmap(h, q_i8, B200MS_I8, n_rows, kTileM, &tq)) return e;
   for (int base = 0; base < n_mtiles;) {
     const int rem = n_mtiles - base;
     int nm = 1;
     while (nm < rem && nm < 4) nm <<= 1;
     int e;
     switch (nm) {
-      case 1: e = launch_b1_umma_one<1>(h, h->tmap_q, tok_const, base, n_groups_real, group_scores, ld, s); break;
-      case 2: e = launch_b1_umma_one<2>(h, h->tmap_q, tok_const, base, n_groups_real, group_scores, ld, s); break;
-      default: e = launch_b1_umma_one<4>(h, h->tmap_q, tok_const, base, n_groups_real, group_scores, ld, s); break;
+      case 1: e = launch_b1_umma_one<1>(h, *tq, tok_const, base, n_groups_real, group_scores, ld, s); break;
+      case 2: e = launch_b1_umma_one<2>(h, *tq, tok_const, base, n_groups_real, group_scores, ld, s); break;
+      default: e = launch_b1_umma_one<4>(h, *tq, tok_const, base, n_groups_real, group_scores, ld, s); break;
     }
     if (e) return e;
     base += nm;

@@ -53,7 +53,6 @@ constexpr uint32_t kRmRawGroupBytes = kRmGroupTiles * kRmRawTile;
 constexpr int kRmMaxStages = 14;      // TMA kinds: 16 / 32 KB patch tiles in flight (HBM latency x bandwidth wants > 128 KB per SM)
 constexpr int kRmARing = 8;           // KIND 3: expanded A tiles in TMEM (32 columns each, columns [256, 512))
 constexpr uint32_t kRmAColBase = 256;
-constexpr uint32_t kRmBarBytes = 2048;  // full[16] empty[16] tfull[8] tempty[8] qfull rfull[64] rempty[64] + TMEM slot
 
 __device__ __forceinline__ void bulk_load_1d(void* dst, const void* src, uint32_t bytes, uint64_t* bar, uint64_t policy) {
   asm volatile(
@@ -282,7 +281,7 @@ maxsim_rowm_kernel(const __grid_constant__ CUtensorMap tmap_rows, const __grid_c
                    const uint8_t* __restrict__ raw_rows, int64_t n_rows, const int32_t* __restrict__ tok_const,
                    const int32_t* __restrict__ chunk_page, const int32_t* __restrict__ unit_start,
                    const int32_t* __restrict__ unit_end, int n_units, int n_groups_real, const uint32_t* __restrict__ clamp_bits,
-                   typename RmTraits<KIND>::Acc* __restrict__ group_scores, int64_t ld, int num_stages, int fast_path) {
+                   typename RmTraits<KIND>::Acc* __restrict__ group_scores, int64_t ld, int num_stages) {
   using T = RmTraits<KIND>;
   using K = typename T::K;
   using Acc = typename T::Acc;
@@ -299,7 +298,7 @@ maxsim_rowm_kernel(const __grid_constant__ CUtensorMap tmap_rows, const __grid_c
   uint8_t* smem_rawring = smem_st;
   int* pm = reinterpret_cast<int*>(smem_st + (KIND == 3 ? size_t(kRmRawGroups) * kRmRawGroupBytes : size_t(num_stages) * K::kTileBytes));
   int* cnt = pm + NG * kRmSlots * 32;  // pm: [NG][kRmSlots][32] per-token maxima; cnt: [kRmSlots] chunks merged so far
-  uint64_t* bars = reinterpret_cast<uint64_t*>(cnt + kRmSlots);
+  uint64_t* bars = reinterpret_cast<uint64_t*>(cnt + kRmSlots);  // kBarrierBytes: the arrays below + TMEM slot + tile count
   uint64_t* full = bars;            // [num_stages] A tile ready for the MMA  (TMA bytes | KIND 3: 4 expander warps)
   uint64_t* empty = bars + 16;      // [num_stages] MMA done with the stage
   uint64_t* tfull = bars + 32;      // [kAcc]       MMA -> epilogue
@@ -548,7 +547,7 @@ maxsim_rowm_kernel(const __grid_constant__ CUtensorMap tmap_rows, const __grid_c
           flush();
           cp = -1;
         }
-        if (fast_path && vmask == 0xffffffffu && (cmask & ~1u) == 0u) {
+        if (vmask == 0xffffffffu && (cmask & ~1u) == 0u) {
           // fast path: 8 whole tiles of ONE page (it may begin at this block's first chunk -- 1024-row pages are exactly one
           // block): at most one adoption, then four owned tiles without bookkeeping
           if (last_pg != cp) adopt(last_pg, 0u);
@@ -647,47 +646,26 @@ maxsim_rowm_kernel(const __grid_constant__ CUtensorMap tmap_rows, const __grid_c
       if (lane == 0) mbar_arrive(&full[stage]);
     }
   }
-
-  tc_fence_before();
-  __syncthreads();
-  if (warp == 2) {
-    tc_fence_after();
-    tmem_dealloc_512(tmem_base);
-  }
+  tile_teardown<false>(warp, tmem_base);
 }
 
+// Resident shared memory: the query panels (1 KB aligned), the [NG][kRmSlots][32] maxima table and the kRmSlots counters.
+// KIND 0-2 stream patch tiles through up to kRmMaxStages stages; KIND 3 adds the raw-bit ring and its kRmARing stages are
+// A tiles in TMEM.
 template <int KIND, int NG>
 static int launch_rowm_one(b200ms_t* h, const CUtensorMap& tq, const int32_t* tok_const, int n_groups_real,
                            const uint32_t* clamp_bits, void* scores, int64_t ld, cudaStream_t s) {
   using T = RmTraits<KIND>;
   using K = typename T::K;
   const Corpus& c = h->corpus;
-  const uint32_t q_bytes = ((K::kPanels * NG * 4096u) + 1023u) & ~1023u;
-  const uint32_t fixed = 1024 + q_bytes + NG * kRmSlots * 32 * 4 + kRmSlots * 4 + kRmBarBytes;
-  int stages;
-  uint32_t smem;
-  if (KIND == 3) {  // shared memory holds the raw-bit ring only; the A tiles live in TMEM
-    stages = kRmARing;
-    smem = fixed + kRmRawGroups * kRmRawGroupBytes;
-  } else {
-    stages = int((kSmemLimit - fixed) / K::kTileBytes);
-    if (stages > kRmMaxStages) stages = kRmMaxStages;
-    if (stages < 2) return set_error(h, B200MS_EINVAL, "maxsim_rowm: not enough shared memory for 2 stages");
-    smem = fixed + uint32_t(stages) * K::kTileBytes;
-  }
-  auto kern = maxsim_rowm_kernel<KIND, NG>;
-  if (int e = ensure_smem(h, reinterpret_cast<const void*>(kern), int(smem), "cudaFuncSetAttribute(maxsim_rowm)")) return e;
-  int grid = h->max_ctas > 0 ? h->max_ctas : h->num_sms;
-  if (grid > c.n_units) grid = c.n_units;
-  if (grid < 1) return B200MS_OK;
+  uint32_t resident = ((K::kPanels * NG * 4096u + 1023u) & ~1023u) + NG * kRmSlots * 32 * 4 + kRmSlots * 4;
+  if (KIND == 3) resident += kRmRawGroups * kRmRawGroupBytes;
   const int32_t* us = static_cast<const int32_t*>(h->unit_start.p);
-  kern<<<grid, T::kThreads, smem, s>>>(c.tmap, tq, static_cast<const uint8_t*>(c.rows), c.n_rows, tok_const,
-                                      static_cast<const int32_t*>(h->chunk_page.p), us, us + 1, c.n_units,
-                                      n_groups_real, clamp_bits,
-                                      static_cast<typename T::Acc*>(scores), ld, stages,
-                                      h->rowm_fast_path != 0);
-  h->launches++;
-  return check_cuda(h, cudaGetLastError(), "launch maxsim_rowm");
+  return launch_persistent(h, maxsim_rowm_kernel<KIND, NG>, "maxsim_rowm", T::kThreads, resident,
+                           KIND == 3 ? 0u : K::kTileBytes, KIND == 3 ? kRmARing : kRmMaxStages, c.n_units, s, c.tmap, tq,
+                           static_cast<const uint8_t*>(c.rows), c.n_rows, tok_const,
+                           static_cast<const int32_t*>(h->chunk_page.p), us, us + 1, c.n_units, n_groups_real, clamp_bits,
+                           static_cast<typename T::Acc*>(scores), ld);
 }
 
 // Full scan of the attached corpus with n_groups_real <= kRowmMaxGroups 32-token query groups.  q_packed: the packed query
@@ -718,27 +696,21 @@ int launch_score_rowm(b200ms_t* h, const void* q_packed, int n_groups_real, cons
   } else if (!c.has_tmap) {
     return set_error(h, B200MS_ESTATE, "score: corpus has no TMA descriptor");
   }
-  const int box = 32 * ng;
-  if (h->tmap_qn_base != q_rows || h->tmap_qn_dtype != q_dtype || h->tmap_qn_rows != n_q_rows || h->tmap_qn_box != box) {
-    if (int e = make_tmap_rows(h, &h->tmap_qn, q_rows, q_dtype, int64_t(n_q_rows), box)) return e;
-    h->tmap_qn_base = q_rows;
-    h->tmap_qn_dtype = q_dtype;
-    h->tmap_qn_rows = n_q_rows;
-    h->tmap_qn_box = box;
-  }
+  const CUtensorMap* tq;  // the query is the N operand: a 32*NG-row box
+  if (int e = query_tmap(h, q_rows, q_dtype, n_q_rows, 32 * ng, &tq)) return e;
   switch (c.dtype) {
     case B200MS_BF16:
-      return ng == 1 ? launch_rowm_one<0, 1>(h, h->tmap_qn, tok_const, n_groups_real, clamp_bits, group_scores, ld, s)
-                     : launch_rowm_one<0, 2>(h, h->tmap_qn, tok_const, n_groups_real, clamp_bits, group_scores, ld, s);
+      return ng == 1 ? launch_rowm_one<0, 1>(h, *tq, tok_const, n_groups_real, clamp_bits, group_scores, ld, s)
+                     : launch_rowm_one<0, 2>(h, *tq, tok_const, n_groups_real, clamp_bits, group_scores, ld, s);
     case B200MS_I8:
-      return ng == 1 ? launch_rowm_one<1, 1>(h, h->tmap_qn, tok_const, n_groups_real, clamp_bits, group_scores, ld, s)
-                     : launch_rowm_one<1, 2>(h, h->tmap_qn, tok_const, n_groups_real, clamp_bits, group_scores, ld, s);
+      return ng == 1 ? launch_rowm_one<1, 1>(h, *tq, tok_const, n_groups_real, clamp_bits, group_scores, ld, s)
+                     : launch_rowm_one<1, 2>(h, *tq, tok_const, n_groups_real, clamp_bits, group_scores, ld, s);
     case B200MS_F8:
-      return ng == 1 ? launch_rowm_one<2, 1>(h, h->tmap_qn, tok_const, n_groups_real, clamp_bits, group_scores, ld, s)
-                     : launch_rowm_one<2, 2>(h, h->tmap_qn, tok_const, n_groups_real, clamp_bits, group_scores, ld, s);
+      return ng == 1 ? launch_rowm_one<2, 1>(h, *tq, tok_const, n_groups_real, clamp_bits, group_scores, ld, s)
+                     : launch_rowm_one<2, 2>(h, *tq, tok_const, n_groups_real, clamp_bits, group_scores, ld, s);
     case B200MS_B1:  // one group only: with 640 threads the two-group epilogue does not fit the 96-register budget
       if (ng != 1) return set_error(h, B200MS_EINVAL, "maxsim_rowm: sign-bit corpora take one query group");
-      return launch_rowm_one<3, 1>(h, h->tmap_qn, tok_const, n_groups_real, nullptr, group_scores, ld, s);
+      return launch_rowm_one<3, 1>(h, *tq, tok_const, n_groups_real, nullptr, group_scores, ld, s);
     default:
       return set_error(h, B200MS_ESTATE, "score: corpus dtype has no row-major-M scorer");
   }

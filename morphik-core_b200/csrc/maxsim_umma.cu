@@ -344,10 +344,10 @@ static int launch_kind(b200ms_t* h, const UnitPlan& up, const CUtensorMap& tq, i
   return B200MS_OK;
 }
 
-// m_tile_lo / m_tile_hi: score only query tiles [m_tile_lo, m_tile_hi) (hi < 0: all) -- the batched rerank walks the query
-// tiles one launch at a time, each against its own candidate units.
+// m_tile >= 0: score only that query tile, on the single-tile kernel -- the batched rerank launches each query tile against
+// its own (short) candidate lists.
 int launch_score_umma(b200ms_t* h, const UnitPlan* plan, const void* q_packed, int n_groups_real, void* group_scores,
-                      int64_t ld, cudaStream_t s, int m_tile_lo, int m_tile_hi) {
+                      int64_t ld, cudaStream_t s, int m_tile) {
   const Corpus& c = h->corpus;
   UnitPlan up;
   if (plan) {
@@ -361,29 +361,19 @@ int launch_score_umma(b200ms_t* h, const UnitPlan* plan, const void* q_packed, i
   if (!c.has_tmap) return set_error(h, B200MS_ESTATE, "score: corpus has no TMA descriptor");
   const int n_groups_padded = (n_groups_real + 3) & ~3;
   const int n_mtiles = n_groups_padded / 4;
-  const int n_q_rows = n_groups_padded * kGroup;
-  if (h->tmap_q_base != q_packed || h->tmap_q_dtype != c.dtype || h->tmap_q_rows != n_q_rows) {
-    if (int e = make_tmap_rows(h, &h->tmap_q, q_packed, c.dtype, int64_t(n_q_rows), kTileM)) return e;
-    h->tmap_q_base = q_packed;
-    h->tmap_q_dtype = c.dtype;
-    h->tmap_q_rows = n_q_rows;
-  }
-  if (m_tile_hi >= 0) {  // one explicit tile range: the single-tile kernel per tile (candidate lists are short)
-    for (int m = m_tile_lo; m < m_tile_hi && m < n_mtiles; ++m) {
-      int e;
-      switch (kind_of_dtype(c.dtype)) {
-        case 0: e = launch_one<0, 1>(h, up, h->tmap_q, m, n_groups_real, group_scores, ld, s); break;
-        case 1: e = launch_one<1, 1>(h, up, h->tmap_q, m, n_groups_real, group_scores, ld, s); break;
-        default: e = launch_one<2, 1>(h, up, h->tmap_q, m, n_groups_real, group_scores, ld, s); break;
-      }
-      if (e) return e;
+  const CUtensorMap* tq;
+  if (int e = query_tmap(h, q_packed, c.dtype, n_groups_padded * kGroup, kTileM, &tq)) return e;
+  if (m_tile >= 0) {
+    switch (kind_of_dtype(c.dtype)) {
+      case 0: return launch_one<0, 1>(h, up, *tq, m_tile, n_groups_real, group_scores, ld, s);
+      case 1: return launch_one<1, 1>(h, up, *tq, m_tile, n_groups_real, group_scores, ld, s);
+      default: return launch_one<2, 1>(h, up, *tq, m_tile, n_groups_real, group_scores, ld, s);
     }
-    return B200MS_OK;
   }
   switch (kind_of_dtype(c.dtype)) {
-    case 0: return launch_kind<0>(h, up, h->tmap_q, n_groups_real, n_mtiles, group_scores, ld, s);
-    case 1: return launch_kind<1>(h, up, h->tmap_q, n_groups_real, n_mtiles, group_scores, ld, s);
-    case 2: return launch_kind<2>(h, up, h->tmap_q, n_groups_real, n_mtiles, group_scores, ld, s);
+    case 0: return launch_kind<0>(h, up, *tq, n_groups_real, n_mtiles, group_scores, ld, s);
+    case 1: return launch_kind<1>(h, up, *tq, n_groups_real, n_mtiles, group_scores, ld, s);
+    case 2: return launch_kind<2>(h, up, *tq, n_groups_real, n_mtiles, group_scores, ld, s);
     default: return set_error(h, B200MS_ESTATE, "score: corpus dtype has no tcgen05 scorer");
   }
 }

@@ -365,13 +365,12 @@ template <int KIND, int NM>
 static int launch_pair(b200ms_t* h, const UnitPlan& up, const CUtensorMap& tq, int m_tile_base, int n_groups_real,
                        void* scores, int64_t ld, cudaStream_t s) {
   using K = Kind<KIND>;
-  const uint32_t avail = kSmemLimit - 1024 - kBarrierBytes - NM * K::kTileBytes;
-  int stages = int(avail / K::kTileBytes);
-  if (stages > 8) stages = 8;
-  if (stages < 2) return set_error(h, B200MS_EINVAL, "maxsim_umma_pair: not enough shared memory for 2 stages");
-  const uint32_t smem = 1024 + NM * K::kTileBytes + uint32_t(stages) * K::kTileBytes + kBarrierBytes;
   const auto launch = [&](auto kern, const char* name, int want) {
-    if (int e = ensure_smem(h, reinterpret_cast<const void*>(kern), int(smem), name)) return e;
+    int stages;
+    uint32_t smem;
+    if (int e = size_stage_ring(h, reinterpret_cast<const void*>(kern), name, NM * K::kTileBytes, K::kTileBytes, 8, &stages,
+                                &smem))
+      return e;
     if (up.n_units < 1) return int(B200MS_OK);
     if (!pairs_schedulable(h, reinterpret_cast<const void*>(kern), smem)) return B200MS_EUNSUPPORTED_PAIR;
     int grid = (h->max_ctas > 0 ? h->max_ctas : h->num_sms) & ~1;  // whole pairs

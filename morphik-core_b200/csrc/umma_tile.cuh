@@ -1,5 +1,7 @@
 // umma_tile.cuh -- tile geometry, pipeline pieces and accumulator helpers shared by the query-as-M tcgen05 MaxSim kernels
-// (maxsim_umma.cu: one CTA per SM; maxsim_umma_pair.cu: CTA pairs, cta_group::2; maxsim_b1_umma.cu: 1-bit rows).
+// (maxsim_umma.cu: one CTA per SM; maxsim_umma_pair.cu: CTA pairs, cta_group::2; maxsim_b1_umma.cu: 1-bit rows).  The
+// lone-query kernel (maxsim_rowm.cu) also uses the teardown and launch_persistent, the FDE scan (fde.cu) the CTA layout and
+// lifetime pieces and launch_persistent.
 #pragma once
 #include <type_traits>
 
@@ -267,16 +269,29 @@ struct UnitWalk {
 };
 
 // ---------------------------------------------------------------------------------------------- host side
-// Persistent one-CTA launch: a ring of as many tile_bytes stages as fit beside resident_bytes in the 227 KB opt-in (at most
-// max_stages, at least 2), grid = one CTA per SM (or max_ctas), at most one per unit.  num_stages is the kernel's last argument.
+// Stage ring of a kernel whose dynamic shared memory is [1024-aligned] resident_bytes | stages x tile_bytes | kBarrierBytes:
+// as many stages as fit the 227 KB opt-in, at most max_stages, at least 2.  tile_bytes = 0: the stages hold no shared memory
+// (maxsim_rowm_kernel<3> keeps its A tiles in TMEM) and there are max_stages of them.  Raises the kernel's shared-memory limit.
+static int size_stage_ring(b200ms_t* h, const void* kern, const char* name, uint32_t resident_bytes, uint32_t tile_bytes,
+                           int max_stages, int* stages, uint32_t* smem) {
+  int n = tile_bytes ? int((kSmemLimit - 1024 /*align*/ - kBarrierBytes - resident_bytes) / tile_bytes) : max_stages;
+  if (n > max_stages) n = max_stages;
+  if (n < 2) return set_error(h, B200MS_EINVAL, std::string(name) + ": not enough shared memory for 2 stages");
+  *stages = n;
+  *smem = 1024 + resident_bytes + uint32_t(n) * tile_bytes + kBarrierBytes;
+  return ensure_smem(h, kern, int(*smem), name);
+}
+
+// Persistent one-CTA launch on a size_stage_ring ring, grid = one CTA per SM (or max_ctas), at most one per unit.
+// num_stages is the kernel's last argument.
 template <typename... Params, typename... Args>
 static int launch_persistent(b200ms_t* h, void (*kern)(Params...), const char* name, int threads, uint32_t resident_bytes,
                              uint32_t tile_bytes, int max_stages, int n_units, cudaStream_t s, Args... args) {
-  int stages = int((kSmemLimit - 1024 /*align*/ - kBarrierBytes - resident_bytes) / tile_bytes);
-  if (stages > max_stages) stages = max_stages;
-  if (stages < 2) return set_error(h, B200MS_EINVAL, std::string(name) + ": not enough shared memory for 2 stages");
-  const uint32_t smem = 1024 + resident_bytes + uint32_t(stages) * tile_bytes + kBarrierBytes;
-  if (int e = ensure_smem(h, reinterpret_cast<const void*>(kern), int(smem), name)) return e;
+  int stages;
+  uint32_t smem;
+  if (int e = size_stage_ring(h, reinterpret_cast<const void*>(kern), name, resident_bytes, tile_bytes, max_stages, &stages,
+                              &smem))
+    return e;
   int grid = h->max_ctas > 0 ? h->max_ctas : h->num_sms;
   if (grid > n_units) grid = n_units;
   if (grid < 1) return B200MS_OK;

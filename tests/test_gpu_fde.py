@@ -168,7 +168,7 @@ def test_upstream_knobs_fill_empty_partitions_and_final_projection():
     assert ((np.abs(q).sum(axis=2) > 0).sum(axis=1) <= 3).all()  # queries are never filled
 
 
-@pytest.mark.parametrize("n_q", [1, 3, 16, 17, 32, 100, 130])
+@pytest.mark.parametrize("n_q", [1, 3, 16, 17, 32, 50, 80, 100, 130])
 def test_fde_scan_tensor_path_matches_simt_and_numpy(n_q):
     """fde_scan_umma_kernel (pages = M, bf16 hi/lo queries = N, the matrix read once per 128 queries) against the SIMT scan
     and numpy: partial last tile, every accumulator-width class (16 / 32 / .. / 128 columns per half), > 128 queries."""
